@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's step restated on the host CPU
+    python bench.py --dump-outputs DIR ...    # also write the last timed step's results to DIR/<name>.npy
 
 One "step" = one iteration of the reference's hot loop `sess.run([train_op, global_step])`
 (/root/reference/scripts/runners.py:231-232) on one synthetic batch.  Rank 0 prints ONE JSON line.
@@ -212,6 +213,28 @@ def flush_l2(buf):
     buf.add_(1)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(eng, out_dir):
+    """What a caller of the timed step receives from it: the loss terms [loss, nll, kl_div_z, nent] and every parameter as
+    Adam left it, float32, one DIR/<name>.npy each ("/" in a variable name becomes ".").  The step they come from starts from
+    the engine's seeded initial state (run_gpu_arm restores it, untimed, before the last timed step) on the seeded batch, with
+    noise keyed by seed and step: the batch is reduce-added across CTAs in no fixed order, so steps that build on earlier
+    ones would carry that rounding forward, amplified by Adam.  Two runs, or two builds, with the same arguments can
+    therefore be compared array for array."""
+    import numpy as np
+    arrays = {"loss_terms": eng.loss_buf}
+    arrays.update(("param." + name.replace("/", "."), v) for name, v in eng.parameters().items())
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_gpu_arm(args, w):
     import torch.distributed as dist
     import gmvae_b200
@@ -230,6 +253,7 @@ def run_gpu_arm(args, w):
                             max_batch=B, device=local, seed=1234)   # same weights on every rank; noise is keyed by rank
     if world > 1:
         eng.init_data_parallel()
+    init_state = eng.state_dict() if args.dump_outputs else None
 
     x_host = synthetic_images(B, 1234 + rank).pin_memory()
     x_dev = x_host.to(dev)
@@ -273,6 +297,8 @@ def run_gpu_arm(args, w):
             sampler.mark()
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
         for i in range(args.steps):
+            if init_state is not None and i == args.steps - 1:
+                eng.load_state_dict(init_state)   # the dumped step starts from the seeded initial state (untimed)
             flush_l2(l2_buf)                      # evict the previous step's tensors from L2 (untimed)
             ev[i][0].record(side)
             step()
@@ -283,6 +309,8 @@ def run_gpu_arm(args, w):
         dev_ms = sum(step_ms)
         med_ms = step_ms[len(step_ms) // 2]
         loss_terms = eng.loss_buf.cpu().tolist()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(eng, args.dump_outputs)
 
         # ---- per-kernel-class device time: CUDA events after every launch of 3 eager steps --------
         prof_steps = 3
@@ -426,7 +454,12 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="override the per-GPU batch")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss terms and parameters to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     w = WORKLOADS[args.workload]
     if args.impl == "reference":

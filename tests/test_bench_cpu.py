@@ -60,3 +60,11 @@ def test_reference_arm_prints_the_contract_line():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
                        capture_output=True, text=True, timeout=120, env=dict(os.environ, RANK="1", WORLD_SIZE="2"))
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_rejected_arguments(tmp_path):
+    for extra, msg in ((["--steps", "0"], "--steps must be at least 1"),
+                       (["--impl", "reference", "--dump-outputs", str(tmp_path / "d")], "--dump-outputs applies to the GPU arm")):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and msg in r.stderr and r.stdout == "", (extra, r.stderr[-2000:])
+    assert not (tmp_path / "d").exists()
