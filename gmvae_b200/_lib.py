@@ -22,7 +22,7 @@ class Config(C.Structure):
         ("num_hidden", C.c_int32), ("hidden_sizes", C.c_int32 * MAX_HIDDEN), ("max_batch", C.c_int32),
         ("sigma_min", C.c_float), ("raw_sigma_bias", C.c_float), ("gen_bias_init", C.c_float),
         ("temperature", C.c_float), ("learning_rate", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float),
-        ("epsilon", C.c_float), ("device", C.c_int32), ("reserved", C.c_int32 * 7),
+        ("epsilon", C.c_float), ("device", C.c_int32), ("deterministic", C.c_int32), ("reserved", C.c_int32 * 6),
     ]
 
 

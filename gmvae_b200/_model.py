@@ -16,14 +16,16 @@ class _EngineBacked:
         raise NotImplementedError
 
     def _init_backing(self, precision: str = "bf16", objective: str = "reference", learning_rate: float = 1e-3,
-                      max_batch: Optional[int] = None, device: Optional[int] = None):
+                      max_batch: Optional[int] = None, device: Optional[int] = None, deterministic: bool = False):
         self._precision, self._objective = precision, objective
+        self._deterministic = deterministic
         self._learning_rate, self._max_batch, self._device = learning_rate, max_batch, device
         self._engine: Optional[Engine] = None
 
     def configure(self, precision: Optional[str] = None, objective: Optional[str] = None,
-                  learning_rate: Optional[float] = None, max_batch: Optional[int] = None, device: Optional[int] = None):
-        """Additive knobs with no reference counterpart (precision / objective / optimiser lr)."""
+                  learning_rate: Optional[float] = None, max_batch: Optional[int] = None, device: Optional[int] = None,
+                  deterministic: Optional[bool] = None):
+        """Additive knobs with no reference counterpart (precision / objective / optimiser lr / bitwise-reproducible steps)."""
         if self._engine is not None:
             raise RuntimeError("configure() must be called before the first run_model()")
         if precision is not None: self._precision = precision
@@ -31,6 +33,7 @@ class _EngineBacked:
         if learning_rate is not None: self._learning_rate = learning_rate
         if max_batch is not None: self._max_batch = max_batch
         if device is not None: self._device = device
+        if deterministic is not None: self._deterministic = bool(deterministic)
         return self
 
     def engine(self, batch: Optional[int] = None) -> Engine:
@@ -41,7 +44,7 @@ class _EngineBacked:
             kw = self._engine_kwargs()
             self._engine = Engine(precision=self._precision, objective=self._objective, max_batch=int(mb),
                                   learning_rate=self._learning_rate, device=self._device,
-                                  seed=self.random_seed, **kw)
+                                  seed=self.random_seed, deterministic=self._deterministic, **kw)
         return self._engine
 
     def _run(self, images, targets, eps, gumbel_u) -> torch.Tensor:

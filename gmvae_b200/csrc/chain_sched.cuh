@@ -42,6 +42,8 @@ struct alignas(16) ChainJob {
                                      // an in-order walker cannot step over a long weight-gradient tile to the chain tile queued behind it
   int share;                         // quad mode: the two pair tiles of a double tile cover the same rows (tiles_n even): A is loaded once, multicast
   int fuse;                          // EK_STORE_F32 jobs with N <= 16: a y head applied to the row in the epilogue (EK_ROWS_Y_FWD / _BWD), 0 = none
+  int zslice;                        // EK_ATOMIC, deterministic mode: tile of k-split z STORES its partial into slice z of the 3-D map d
+                                     // ([splits][M][ld], det_slice_index) instead of reduce-adding into the gradient buffer
   alignas(16) unsigned char epi2[CHAIN_EPI2_BYTES];   // its parameters (RowsYFwd / RowsYBwd)
 };
 // Tile l of a job -> (k-split z, row block mb, first column n0).  n fastest, then m, then k-split.  With J.rot the n-tile index
@@ -100,6 +102,18 @@ inline void chain_job_geometry(ChainJob& J, int M, int N, int block_n, int split
   J.share = (cl == 4 && tiles_n % 2 == 0) ? 1 : 0;
   J.rot = (tiles_n > 1 && N % block_n != 0 && !a_mn) ? 1 : 0;
 }
+// Deterministic mode: where element (m, n) of k-split z of a weight-gradient job lives in its partial buffer, slices of M rows x ld
+// floats (ld = N rounded up to 4: 16-byte rows for TMA).  The tiles store through a 3-D tensor map of this layout (a ragged row block
+// is clipped at M within its own slice); det_reduce_kernel adds slices 0 .. splits-1 of every element in that order.
+GMVAE_SCHED_FN int det_slice_ld(int N) { return (N + 3) / 4 * 4; }
+GMVAE_SCHED_FN long long det_slice_index(int z, int m, int n, int M, int ld) { return ((long long)z * M + m) * ld + n; }
+// The rows / columns tile (z, mb, n0) of a weight-gradient job writes: [r0, r1) x [c0, c1) of slice z (empty for a phantom half)
+GMVAE_SCHED_FN void det_tile_region(const ChainJob& J, int mb, int n0, int& r0, int& r1, int& c0, int& c1) {
+  r0 = mb * SCHED_BLOCK_M; r1 = r0 + SCHED_BLOCK_M < J.M ? r0 + SCHED_BLOCK_M : J.M;
+  c0 = n0; c1 = n0 + J.block_n < J.N ? n0 + J.block_n : J.N;
+  if (r1 < r0) r1 = r0;
+}
+
 // Row-block counters a job's tiles signal (phantom halves / phantom pair tiles signal counters nobody waits for)
 inline int chain_job_counters(int M, int cl) {
   const int tiles_m = (M + SCHED_BLOCK_M - 1) / SCHED_BLOCK_M;

@@ -128,7 +128,23 @@ __device__ __forceinline__ float block_sum(float v, float* scratch) {
 // and summed in double by the finalising kernel: thousands of same-sized addends into ONE fp32
 // accumulator round in a correlated way (measured: 1.6e-4 relative on the 16 384-sample KAT).
 enum { ACC_NLL = 0, ACC_KL = 32, ACC_NENT = 64, ACC_PER_TERM = 32, ACC_SLOTS = 96 };
+// Deterministic mode (gmvae_config::deterministic): sums whose addends arrive in no fixed order are taken in fixed point, as
+// int64 multiples of 2^-FX_SHIFT.  Integer addition is associative, so the total does not depend on the order of arrival; the
+// reduction step (det_reduce_kernel) converts it to fp32.  Resolution 1.5e-11 per addend.  Sum i lives in fx[2i]; fx[2i + 1]
+// flags an addend that is not finite or beyond +-2^26 (whose fixed-point form would saturate), and the reduction step then
+// writes NaN, as a NaN addend would have made of the default mode's float sum.  A sum of in-range addends beyond +-2^27 wraps
+// unflagged; the sums taken this way (loss terms, VAE_GMP prior gradients: means over the batch) stay far below that.
+enum { FX_SHIFT = 36 };
+__device__ __forceinline__ void fx_add(unsigned long long* fx, int i, float v) {
+  if (fabsf(v) < 67108864.f) atomicAdd(fx + 2 * i, (unsigned long long)__float2ll_rn(v * (float)(1ull << FX_SHIFT)));   // two's complement
+  else atomicOr(fx + 2 * i + 1, 1ull);                                                                                 // also NaN
+}
+// The training step passes the accumulator base with bit 0 set in deterministic mode: it then points at the fixed-point sums
+// above, one per term (index term / ACC_PER_TERM).
+inline float* acc_fixed_tag(unsigned long long* fx) { return reinterpret_cast<float*>(reinterpret_cast<uintptr_t>(fx) | 1u); }
 __device__ __forceinline__ void acc_add(float* acc, int term, float v) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(acc);
+  if (a & 1u) { fx_add(reinterpret_cast<unsigned long long*>(a & ~(uintptr_t)1), term / ACC_PER_TERM, v); return; }
   atomicAdd(acc + term + ((blockIdx.x + (threadIdx.x >> 5)) & (ACC_PER_TERM - 1)), v);
 }
 __device__ __forceinline__ float acc_total(const float* acc, int term) {

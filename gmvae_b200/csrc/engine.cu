@@ -102,6 +102,25 @@ int make_tmap_bf16(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t o
                    uint32_t box_inner, uint32_t box_outer) {
   return make_tmap(out, ptr, 2, inner, outer, outer_stride, box_inner, box_outer, 128);
 }
+// fp32 [slices][outer][inner] with `ld` floats between rows and outer * ld between slices (deterministic mode's weight-gradient
+// partials, chain_sched.cuh det_slice_index); box = {box_inner, box_outer, 1}: a box never crosses into the next slice
+int make_tmap_slices_f32(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t outer, uint64_t slices, uint64_t ld,
+                         uint32_t box_inner, uint32_t box_outer) {
+  EncodeTiledFn fn = get_encode_fn();
+  GM_REQUIRE(fn != nullptr, "cuTensorMapEncodeTiled not available from the driver");
+  GM_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 15) == 0 && ld % 4 == 0, "TMA slices need 16-byte aligned rows");
+  cuuint64_t gdim[3] = {inner, outer, slices};
+  cuuint64_t gstride[2] = {ld * 4, outer * ld * 4};
+  cuuint32_t box[3] = {box_inner, box_outer, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(ptr), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled (slices) failed with CUresult " + std::to_string((int)r));
+    return -3;
+  }
+  return 0;
+}
 }  // namespace tc
 
 // ============================================================================ model description
@@ -221,6 +240,13 @@ struct gmvae_handle {
   FuseReq fuse_next;
   bool last_gemm_chained = false;                 // set by the GEMM dispatch: the last GEMM became a job of the chain
   std::map<const void*, bool> relu_bits_valid;    // hidden activation -> its 1-bit ReLU mask was written this step
+  // deterministic mode (gmvae_config::deterministic): the segments the reduction step of this step sums (det_reduce_kernel) and the
+  // partial rows of the column sums handed out so far (floats of the "det.part" buffer)
+  bool det = false;
+  std::vector<DetSeg> det_segs;
+  std::vector<std::function<int()>> det_colsums;  // column sums of this step, launched after its last chained launch
+  int64_t det_part_next = 0, det_part_cap = 0;    // floats of "det.part" (column-sum partial rows)
+  int64_t det_wg_next = 0, det_wg_cap = 0;        // floats of "det.wg" (weight-gradient k-split slices)
   // graph
   cudaGraphExec_t graph_exec = nullptr;
 
@@ -276,6 +302,10 @@ static void plan_shadows(gmvae_handle* h, Mlp& m) {
     plan_buf(h, "shadow.w." + std::to_string(l.w_off), (size_t)l.in * l.ld_w * 2);
   }
 }
+
+// deterministic mode: row blocks of a bias-gradient column sum (a function of nothing but the shapes)
+constexpr int DET_ROW_BLOCKS = 64;
+static int wgrad_split(const gmvae_handle* h, int in, int out, int M, bool pair, bool quad);
 
 static int plan(gmvae_handle* h) {
   const gmvae_config& c = h->cfg;
@@ -359,6 +389,32 @@ static int plan(gmvae_handle* h) {
     if (c.model == GMVAE_MODEL_GMVAE) { plan_shadows(h, h->encoder_y); plan_shadows(h, h->prior_gmm); }
   }
   plan_buf(h, "infer.acc", ACC_SLOTS * 4);
+  if (c.deterministic) {
+    // one column sum per bias per step, DET_ROW_BLOCKS partial rows each; fixed-point sums of the three loss terms and of the
+    // VAE_GMP prior's gradients
+    int64_t cols = 0;
+    for (const Mlp* m : {&h->decoder, &h->encoder, &h->encoder_y, &h->prior_gmm})
+      for (const Linear& l : m->layers) cols += l.out;
+    h->det_part_cap = cols * DET_ROW_BLOCKS;
+    plan_buf(h, "det.part", (size_t)h->det_part_cap * 4);
+    plan_buf(h, "det.fx", (size_t)(3 + (c.model == GMVAE_MODEL_VAE_GMP ? K + 2 * K * Z : 0)) * 16);
+    // k-split slices of every weight gradient, for max_batch (the split count grows with the batch) in either plan
+    h->det_wg_cap = 0;
+    for (const Mlp* m : {&h->decoder, &h->encoder, &h->encoder_y, &h->prior_gmm})
+      for (size_t i = 0; i < m->layers.size(); ++i) {
+        const Linear& l = m->layers[i];
+        std::vector<int> views{l.in};
+        if (m == &h->encoder && i == 0 && c.model == GMVAE_MODEL_GMVAE) views = {D, K};    // [x, y] W: two weight-gradient jobs
+        for (int in : views) {
+          const int kb = (int)((Bfull + tc::BLOCK_K - 1) / tc::BLOCK_K);
+          int S = 1;
+          for (bool pair : {false, true}) S = std::max(S, wgrad_split(h, in, l.out, (int)Bfull, pair, false));
+          S = std::min(S, kb);
+          h->det_wg_cap += round_up((int)std::min<int64_t>((int64_t)S * in * tc::det_slice_ld(l.out), 1LL << 30), 64);
+        }
+      }
+    plan_buf(h, "det.wg", (size_t)h->det_wg_cap * 4);
+  }
   h->chain_counter_cap = 64 * (int)((Bfull + 127) / 128 + 2);
   plan_buf(h, "chain.counters", (size_t)h->chain_counter_cap * 4);
   return 0;
@@ -619,10 +675,15 @@ static int chain_add(gmvae_handle* h, const tc::Operand& A1, const tc::Operand& 
   // epilogue I/O through TMA: boxes of 32 rows x 64 bytes (one patch of the kernel)
   const ChainIO io = chain_io(epi);
   J.gw = 0; J.c = J.a1; J.d = J.a1;
+  J.zslice = (h->det && tc::epi_kind<Epi>::value == tc::EK_ATOMIC) ? 1 : 0;
+  GM_REQUIRE(!J.zslice || io.out, "deterministic mode: weight-gradient slices need 16-byte rows");
   if (io.out) {
     J.gw = io.elem == 2 ? 2 : 1;
     J.d = h->chain.nmaps++;
-    GM_TRY(tc::make_tmap(&h->chain.maps[J.d], io.out, io.elem, (uint64_t)N, (uint64_t)M, (uint64_t)io.ld, io.elem == 2 ? 32 : 16, 32, 64));
+    if (J.zslice)   // k-split z stores into slice z (lin_wgrad sized the buffer for these splits)
+      GM_TRY(tc::make_tmap_slices_f32(&h->chain.maps[J.d], io.out, (uint64_t)N, (uint64_t)M, (uint64_t)J.num_splits, (uint64_t)io.ld, 16, 32));
+    else
+      GM_TRY(tc::make_tmap(&h->chain.maps[J.d], io.out, io.elem, (uint64_t)N, (uint64_t)M, (uint64_t)io.ld, io.elem == 2 ? 32 : 16, 32, 64));
     if (io.opnd) {
       J.c = h->chain.nmaps++;
       GM_TRY(tc::make_tmap(&h->chain.maps[J.c], io.opnd, 2, (uint64_t)N, (uint64_t)M, (uint64_t)io.ld_opnd, 32, 32, 64));
@@ -777,7 +838,21 @@ static int lin_dgrad(gmvae_handle* h, const TD* dY, int64_t ldy, int M, const Li
   return 0;
 }
 
-// dW[in,out] += A^T[in,M] * dY[M,out]   (grads pre-zeroed; split over the batch, fp32 atomics)
+// Tile width and k-split of a weight-gradient GEMM on the tensor cores: one wave of persistent CTAs (CTA pairs): split the batch
+// so that tiles * split ~ number of SMs (pairs), keeping at least 4 k-blocks (256 samples) per split.
+// (with the walker partition a job is two rounds of the weight-gradient pairs: same tiles, same split)
+// (measured at cfg4, tiles x splits as a multiple of the walkers: 0.34 / 0.5 / 0.75 / 1 / 2 / 3 / 4 -> 0.386 / 0.356 / 0.348 / 0.347 / 0.376 /
+// 0.395 / 0.419 ms: shorter tiles pay the reduce-add epilogue more often, longer ones leave pairs without a tile)
+static int wgrad_bn(const gmvae_handle* h, int out) { return out <= 64 ? 64 : (out <= 128 || (h->debug_flags & DBG_BN128)) ? 128 : 256; }
+static int wgrad_split(const gmvae_handle* h, int in, int out, int M, bool pair, bool quad) {
+  const int bn = wgrad_bn(h, out);
+  const int tiles = pair ? ((in + 255) / 256) * ((out + bn - 1) / bn) : ((in + 127) / 128) * ((out + bn - 1) / bn);
+  const int kb = (M + tc::BLOCK_K - 1) / tc::BLOCK_K;
+  const int walkers = quad ? h->max_quads : pair ? tc::num_sms() / 2 : tc::num_sms(), units = quad ? (tiles + 1) / 2 : tiles;   // quad: 4-CTA clusters, double tiles
+  return std::max(1, std::min(std::max(1, kb / 4), walkers / units));
+}
+
+// dW[in,out] += A^T[in,M] * dY[M,out]   (grads pre-zeroed; split over the batch, fp32 atomics; deterministic mode: k-split slices)
 template <typename TA, typename TD>
 static int lin_wgrad(gmvae_handle* h, const TA* A, int64_t lda, const TD* dY, int64_t ldy, int M, const LinView& L,
                      cudaStream_t st) {
@@ -787,25 +862,31 @@ static int lin_wgrad(gmvae_handle* h, const TA* A, int64_t lda, const TD* dY, in
               aligned16(A) && aligned16(dY);
     if (ok) {
       tc::Operand a{A, lda, kpad(L.in, lda), M}, b{dY, ldy, kpad(L.out, ldy), M};
-      const int bn = L.out <= 64 ? 64 : (L.out <= 128 || (h->debug_flags & DBG_BN128)) ? 128 : 256;
+      const int bn = wgrad_bn(h, L.out);
       const bool pair = h->chain_on && h->chain_pair;
-      const int tiles = pair ? ((L.in + 255) / 256) * ((L.out + bn - 1) / bn) : ((L.in + 127) / 128) * ((L.out + bn - 1) / bn);
-      const int kb = (M + tc::BLOCK_K - 1) / tc::BLOCK_K;
-      // one wave of persistent CTAs (CTA pairs): split the batch so that tiles * split ~ number of SMs (pairs),
-      // keeping at least 4 k-blocks (256 samples) per split
-      const bool quad = pair && h->chain_quad;       // walkers: 4-CTA clusters taking double tiles
-      const int walkers = quad ? h->max_quads : pair ? tc::num_sms() / 2 : tc::num_sms(), units = quad ? (tiles + 1) / 2 : tiles;
-      // (with the walker partition a job is two rounds of the weight-gradient pairs: same tiles, same split)
-      // (measured at cfg4, tiles x splits as a multiple of the walkers: 0.34 / 0.5 / 0.75 / 1 / 2 / 3 / 4 -> 0.386 / 0.356 / 0.348 / 0.347 / 0.376 /
-      // 0.395 / 0.419 ms: shorter tiles pay the reduce-add epilogue more often, longer ones leave pairs without a tile)
-      int split = std::max(1, std::min(std::max(1, kb / 4), walkers / units));
+      const int split = wgrad_split(h, L.in, L.out, M, pair, pair && h->chain_quad);
       if (h->chain_on) {
+        EpiAtomicAdd e = epi;
+        if (h->det) {
+          // the k-splits store their partials into slices of this job's buffer (chain_add: a 3-D tensor map); the reduction step
+          // adds slices 0 .. S-1 of every element in that order
+          const int kb = (M + tc::BLOCK_K - 1) / tc::BLOCK_K, per = (kb + split - 1) / split, S = (kb + per - 1) / per;
+          const int ld = tc::det_slice_ld(L.out);
+          const int64_t need = round_up((int)std::min<int64_t>((int64_t)S * L.in * ld, 1LL << 30), 64);
+          GM_REQUIRE(h->det_wg_next + need <= h->det_wg_cap && (int)h->det_segs.size() < DET_MAX_SEGS,
+                     "deterministic mode: out of weight-gradient partial space");
+          float* part = h->buf<float>("det.wg") + h->det_wg_next;
+          h->det_wg_next += need;
+          e = EpiAtomicAdd{part, (int64_t)ld};
+          h->det_segs.push_back(DetSeg{L.dw, part, nullptr, (long long)L.in * ld, L.in, L.out, S, L.ldw32, ld, 0});
+        }
         const int saved_part = h->cur_part;
         if (saved_part == 1) h->cur_part = h->part_tail ? 0 : 2;      // weight gradients: their own walkers (the tail: everybody)
-        const int r = chain_add(h, a, b, nullptr, nullptr, L.in, L.out, bn, true, true, split, epi, st);
+        const int r = chain_add(h, a, b, nullptr, nullptr, L.in, L.out, bn, true, true, split, e, st);
         h->cur_part = saved_part;
         return r;
       }
+      GM_REQUIRE(!h->det, "deterministic mode: weight gradients outside the chained kernel");   // (bf16 always chains there)
       GM_TRY(chain_flush(h, st));
       int r = bn == 64    ? tc::launch_gemm_tc<64, true, true, EpiAtomicAdd>(a, b, nullptr, nullptr, L.in, L.out, split, epi, st)
               : bn == 128 ? tc::launch_gemm_tc<128, true, true, EpiAtomicAdd>(a, b, nullptr, nullptr, L.in, L.out, split, epi, st)
@@ -817,6 +898,7 @@ static int lin_wgrad(gmvae_handle* h, const TA* A, int64_t lda, const TD* dY, in
   GM_TRY(chain_flush(h, st));
   const int tiles = ((L.in + SIMT_BM - 1) / SIMT_BM) * ((L.out + SIMT_BN - 1) / SIMT_BN);
   int split = std::max(1, std::min((M + 255) / 256, (4 * 148 + tiles - 1) / tiles));
+  if (h->det) split = 1;
   GM_CHECK_CUDA((launch_gemm_simt<TA, TD, EpiAtomicAdd>(A, 1, lda, dY, ldy, 1, L.in, L.out, M, split, epi, st)));
   GM_LAUNCHED(h, st, PC_SIMT_GEMM);
   return 0;
@@ -826,10 +908,28 @@ template <typename T>
 static int bias_grad(gmvae_handle* h, const T* dY, int64_t ldy, int M, int N, float* db, cudaStream_t st) {
   const int col_blocks = (N + 255) / 256;
   int rows_per_block = std::max(64, (M * col_blocks + 2 * 148 - 1) / (2 * 148));
+  float* part = nullptr;
+  if (h->det) {
+    // DET_ROW_BLOCKS partial rows (row blocks beyond M store zeros), summed in order by the reduction step
+    rows_per_block = std::max(8, (M + DET_ROW_BLOCKS - 1) / DET_ROW_BLOCKS);
+    GM_REQUIRE(h->det_part_next + (int64_t)N * DET_ROW_BLOCKS <= h->det_part_cap && (int)h->det_segs.size() < DET_MAX_SEGS,
+               "deterministic mode: out of partial-sum space");
+    part = h->buf<float>("det.part") + h->det_part_next;
+    h->det_part_next += (int64_t)N * DET_ROW_BLOCKS;
+    h->det_segs.push_back(DetSeg{db, part, nullptr, N, 1, N, DET_ROW_BLOCKS, 0, N, 0});
+    // run after the step's last chained launch (dY stays untouched until the step ends): the chain is not cut here
+    const int rpb = round_up(rows_per_block, 8);
+    h->det_colsums.push_back([=]() -> int {
+      GM_CHECK_CUDA(launch_k(colsum_kernel<T>, dim3(col_blocks, DET_ROW_BLOCKS), dim3(256), 0, st, true, dY, ldy, M, N, rpb, db, part));
+      GM_LAUNCHED(h, st, PC_BIAS_GRAD);
+      return 0;
+    });
+    return 0;
+  }
   rows_per_block = round_up(rows_per_block, 8);
   dim3 grid(col_blocks, (M + rows_per_block - 1) / rows_per_block);
   GM_TRY(chain_flush(h, st));
-  GM_CHECK_CUDA(launch_k(colsum_kernel<T>, grid, dim3(256), 0, st, true, dY, ldy, M, N, rows_per_block, db));
+  GM_CHECK_CUDA(launch_k(colsum_kernel<T>, grid, dim3(256), 0, st, true, dY, ldy, M, N, rows_per_block, db, part));
   GM_LAUNCHED(h, st, PC_BIAS_GRAD);
   return 0;
 }
@@ -884,7 +984,7 @@ static int mlp_backward(gmvae_handle* h, const Mlp& m, const MlpBufs<A>& b, cons
   // issued here but returned, upper layer first, so that the caller can place them where the chain of dependent
   // jobs needs filler work.
   const int nl = (int)m.layers.size();
-  const bool fuse = !(h->debug_flags & DBG_NO_FUSED_COLSUM);
+  const bool fuse = !(h->debug_flags & DBG_NO_FUSED_COLSUM) && !h->det;   // deterministic mode: column sums by bias_grad
   bool bias_done = dout_bias_done;   // bias gradient of the layer whose output gradient we hold
   // Per layer, top down: first the data gradient (the next layer's input, so the chain of dependent
   // GEMMs keeps moving), then the weight gradient of the same layer (its operands are complete by then).
@@ -1076,6 +1176,18 @@ static int forward_encoder(gmvae_handle* h, const uint8_t* x_u8, int B, float in
 template <typename A>
 static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, int Bg, const float* eps_in, const float* u_in, cudaStream_t st);
 
+// Deterministic mode: the step's final sums in a fixed order (det_reduce_kernel), into the bias entries of the gradient buffer,
+// the VAE_GMP prior's gradients and slot 0 of every loss term of the tail -- where the atomics of the default mode put them.
+static int det_reduce(gmvae_handle* h, cudaStream_t st) {
+  DetSegs segs;
+  segs.nseg = (int)h->det_segs.size();
+  long long nmax = 1;
+  for (int i = 0; i < segs.nseg; ++i) { segs.s[i] = h->det_segs[i]; nmax = std::max(nmax, (long long)segs.s[i].rows * segs.s[i].cols); }
+  GM_CHECK_CUDA(launch_k(det_reduce_kernel, dim3((unsigned)std::min(1024LL, (nmax + 255) / 256), segs.nseg), dim3(256), 0, st, true, segs));
+  GM_LAUNCHED(h, st, PC_BIAS_GRAD);
+  return 0;
+}
+
 // Records the tensor-core GEMMs between two head kernels as one chained launch (gemm_chain.cuh).
 template <typename A>
 static int forward_backward_impl(gmvae_handle* h, const uint8_t* x_u8, int B, int Bg, const float* eps_in,
@@ -1126,6 +1238,11 @@ static int forward_backward_impl(gmvae_handle* h, const uint8_t* x_u8, int B, in
   if (h->chain_on) GM_CHECK_CUDA(cudaMemsetAsync(h->chain_counters, 0, (size_t)h->chain_counter_cap * 4, st));
   int r = forward_backward_body<A>(h, x_u8, B, Bg, eps_in, u_in, st);
   if (r == 0) r = chain_flush(h, st);
+  if (h->det) {
+    for (auto& f : h->det_colsums) if (r == 0) r = f();
+    h->det_colsums.clear();
+    if (r == 0) r = det_reduce(h, st);
+  }
   h->chain_on = false; h->chain_pair = false; h->chain_quad = false; h->chain.njobs = 0; h->chain.nmaps = 0;
   return r;
 }
@@ -1145,6 +1262,19 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
   if (!h->grads_clean) GM_CHECK_CUDA(cudaMemsetAsync(h->grads, 0, (size_t)(h->n_params + ACC_SLOTS) * 4, st));
   h->grads_clean = false;
   h->reduced_upto = 0;
+  unsigned long long* fx = h->det ? h->buf<unsigned long long>("det.fx") : nullptr;
+  if (h->det) {
+    const int nfx = 3 + (c.model == GMVAE_MODEL_VAE_GMP ? K + 2 * K * Z : 0);
+    GM_CHECK_CUDA(cudaMemsetAsync(fx, 0, (size_t)nfx * 16, st));
+    acc = acc_fixed_tag(fx);
+    h->det_segs.clear(); h->det_colsums.clear(); h->det_part_next = 0; h->det_wg_next = 0;
+    h->det_segs.push_back(DetSeg{h->grads + h->n_params, nullptr, fx, 0, 3, 1, 0, ACC_PER_TERM, 0, 0});   // slot 0 of each term
+    if (c.model == GMVAE_MODEL_VAE_GMP) {   // fx sums 3 ..: [K mixture logits | K*Z loc | K*Z raw_scale_diag] (gmp_prior_kernel)
+      h->det_segs.push_back(DetSeg{h->grads + h->mix_off, nullptr, fx + 2 * 3, 0, 1, K, 0, 0, 0, 0});
+      h->det_segs.push_back(DetSeg{h->grads + h->loc_off, nullptr, fx + 2 * (3 + K), 0, 1, K * Z, 0, 0, 0, 0});
+      h->det_segs.push_back(DetSeg{h->grads + h->raw_scale_off, nullptr, fx + 2 * (3 + K + K * Z), 0, 1, K * Z, 0, 0, 0, 0});
+    }
+  }
 
   const float* eps = eps_in; const float* u = u_in;
   GM_TRY(forward_encoder<A>(h, x_u8, B, inv_bg, eps, u, acc, st));
@@ -1196,7 +1326,7 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
     GM_CHECK_CUDA(launch_k(gmp_prior_kernel, dim3((B + warps - 1) / warps), dim3(warps * 32), warps * K * sizeof(float), st, true,
                            (const float*)z_f32, (const float*)(h->params + h->loc_off), (const float*)(h->params + h->raw_scale_off),
                            (const float*)(h->params + h->mix_off), B, K, Z, inv_bg, dz_prior, h->grads + h->loc_off,
-                           h->grads + h->raw_scale_off, h->grads + h->mix_off, acc));
+                           h->grads + h->raw_scale_off, h->grads + h->mix_off, acc, fx ? fx + 2 * 3 : nullptr));
     GM_LAUNCHED(h, st, PC_HEADS);
   }
   // decoder: hidden layers, then logits fused with the Bernoulli log-likelihood (and db of that layer)
@@ -1207,7 +1337,7 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
     const A* in = nl == 1 ? z_act : dec.hid[nl - 2];
     const int64_t ldin = nl == 1 ? Zp : hid_ld(nl - 2);
     LinView Ld = view(h, l);
-    dec_bias_fused = !(h->debug_flags & DBG_NO_FUSED_COLSUM) && tc_ok_fwd<A>(h, in, ldin, Ld);
+    dec_bias_fused = !(h->debug_flags & DBG_NO_FUSED_COLSUM) && !h->det && tc_ok_fwd<A>(h, in, ldin, Ld);
     EpiBCE<A> epi{dlogits_x, (int64_t)Dp, h->params + l.b_off, c.gen_bias_init, x_u8, (int64_t)D, 1, nullptr, (double*)nullptr,
                   acc, inv_bg, 0.f, dec_bias_fused ? h->grads + l.b_off : nullptr, h->bf16_mode() ? 1 : 0};
     GM_TRY(lin_fwd<A>(h, in, ldin, B, Ld, epi, st));
@@ -1244,14 +1374,15 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
   bool enc_bias_fused = false;
   {
     int64_t n = (int64_t)B * Z;
-    enc_bias_fused = Z <= 256 && !(h->debug_flags & DBG_NO_FUSED_COLSUM);
-    const bool rows_ok = h->chain_on && h->row_jobs && enc_bias_fused && prior_mode != 1 &&
+    const bool z_cs_ok = Z <= 256 && !(h->debug_flags & DBG_NO_FUSED_COLSUM);
+    enc_bias_fused = z_cs_ok && !h->det;         // deterministic mode: the row job / kernel leaves the column sums to bias_grad
+    const bool rows_ok = h->chain_on && h->row_jobs && z_cs_ok && prior_mode != 1 &&
                          (Z == 4 || Z == 8 || Z == 16 || Z == 32 || Z == 64) && aligned16(eps) && aligned16(enc_out) && aligned16(dz) &&
                          (prior_mode != 2 || aligned16(prior_out));
     if (rows_ok) {
       tc::RowsZBwd prm{enc_out, eps, prior_out, dz, prior_mode, Z, c.raw_sigma_bias, c.sigma_min, inv_bg, reinterpret_cast<bf16*>(d_enc_out),
-                       reinterpret_cast<bf16*>(d_prior_out), Z2p, h->grads + enc_last.b_off,
-                       gm ? h->grads + h->prior_gmm.layers[0].b_off : (float*)nullptr};
+                       reinterpret_cast<bf16*>(d_prior_out), Z2p, enc_bias_fused ? h->grads + enc_last.b_off : (float*)nullptr,
+                       (gm && enc_bias_fused) ? h->grads + h->prior_gmm.layers[0].b_off : (float*)nullptr};
       GM_TRY(chain_add_rows(h, tc::EK_ROWS_Z_BWD, prm, B, {dz, enc_out, prior_out, eps},
                             {{d_enc_out, (size_t)B * Z2p * 2}, {gm ? d_prior_out : nullptr, (size_t)B * Z2p * 2}}, st, 4));
     } else {
@@ -1296,14 +1427,15 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
     const Linear& lp = h->prior_gmm.layers[0];
     LinView Lp = view(h, lp);
     const bool dy_two_seg = tc_ok_dgrad<A>(h, dh0, ld_dh0, Ly) && tc_ok_dgrad<A>(h, d_prior_out, Z2p, Lp) && !(h->debug_flags & DBG_NO_TWO_SEG);
-    const bool ey_bias_fused = !(h->debug_flags & DBG_NO_FUSED_COLSUM);
+    const bool y_cs_ok = !(h->debug_flags & DBG_NO_FUSED_COLSUM);
+    const bool ey_bias_fused = y_cs_ok && !h->det;
     bool yb_fused = false;
     {
       EpiStore<float> e{dy, (int64_t)K, nullptr, nullptr, 0, 0, 1.f};
-      if (dy_two_seg && h->chain_on && h->row_jobs && K <= 16 && Kp <= 16 && ey_bias_fused && !(h->debug_flags & DBG_NO_FUSE_HEADS)) {
+      if (dy_two_seg && h->chain_on && h->row_jobs && K <= 16 && Kp <= 16 && y_cs_ok && !(h->debug_flags & DBG_NO_FUSE_HEADS)) {
         // the backward of the q(y|x) head runs in the epilogue of the dy GEMM; dy itself never reaches memory
         tc::RowsYBwd prm{logits_y, y_f32, nullptr, K, 1.f / c.temperature, inv_bg, reinterpret_cast<bf16*>(dlogits_y), Kp,
-                         h->grads + h->encoder_y.layers[nl - 1].b_off};
+                         ey_bias_fused ? h->grads + h->encoder_y.layers[nl - 1].b_off : (float*)nullptr};
         h->fuse_next = gmvae_handle::FuseReq();
         h->fuse_next.kind = tc::EK_ROWS_Y_BWD;
         memcpy(h->fuse_next.prm, &prm, sizeof(prm));
@@ -1575,6 +1707,15 @@ int gmvae_create(const gmvae_config* cfg, gmvae_handle** out) {
   GM_REQUIRE(cfg->objective == GMVAE_OBJECTIVE_REFERENCE || cfg->model == GMVAE_MODEL_GMVAE, "objective applies to GMVAE only");
   if (cfg->objective == GMVAE_OBJECTIVE_MARGINAL)
     GM_REQUIRE(cfg->num_hidden >= 1 && cfg->latent_size <= 256, "objective=marginal needs at least one hidden layer and latent_size <= 256");
+  GM_REQUIRE(cfg->deterministic == 0 || cfg->deterministic == 1, "deterministic must be 0 or 1");
+  if (cfg->deterministic) {
+    GM_REQUIRE(cfg->objective == GMVAE_OBJECTIVE_REFERENCE, "deterministic mode supports objective=reference only");
+    // the opt-in launch plans are not covered by the guarantee
+    for (const char* v : {"GMVAE_DEBUG_FLAGS", "GMVAE_CHAIN_SPLIT", "GMVAE_CHAIN_QUAD"}) {
+      const char* e = getenv(v);
+      GM_REQUIRE(!e || atoi(e) == 0, std::string("deterministic mode cannot be combined with ") + v);
+    }
+  }
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0) {
@@ -1590,6 +1731,7 @@ int gmvae_create(const gmvae_config* cfg, gmvae_handle** out) {
   DeviceGuard dev_guard(h);
   const char* dbg = getenv("GMVAE_DEBUG_FLAGS");
   h->debug_flags = dbg ? atoi(dbg) : 0;
+  h->det = cfg->deterministic == 1;
   g_use_pdl = !(h->debug_flags & DBG_NO_PDL);
   if (const char* q = getenv("GMVAE_CHAIN_QUAD")) h->quad_opt_in = atoi(q) != 0;
   if (const char* q = getenv("GMVAE_CHAIN_SPLIT")) h->chain_split_opt = atoi(q);

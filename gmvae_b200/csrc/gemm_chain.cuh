@@ -141,6 +141,10 @@ __device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* m, uint32_t
   asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];"
                ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1) : "memory");
 }
+__device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2) {
+  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
+               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src), "r"(c0), "r"(c1), "r"(c2) : "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
@@ -639,8 +643,12 @@ __device__ __forceinline__ void chain_epilogue_job(const ChainJob& J, const CUte
         fence_proxy_async();                                  // generic-proxy writes to the patch -> visible to the bulk store
         __syncwarp();
         if (lane == 0) {
-          if constexpr (KIND == EK_ATOMIC) tma_reduce_add_2d(&maps[J.d], patch, n0 + gcol, mrow0);
-          else tma_store_2d(&maps[J.d], patch, n0 + gcol, mrow0);
+          if constexpr (KIND == EK_ATOMIC) {
+            if (J.zslice) tma_store_3d(&maps[J.d], patch, n0 + gcol, mrow0, z);
+            else tma_reduce_add_2d(&maps[J.d], patch, n0 + gcol, mrow0);
+          } else {
+            tma_store_2d(&maps[J.d], patch, n0 + gcol, mrow0);
+          }
           bulk_commit();
         }
         if constexpr (KIND == EK_RELUMASK || KIND == EK_BCE) {
@@ -862,7 +870,7 @@ __device__ __forceinline__ void chain_rows_job(const ChainJob& J, int* counters,
     for (int col = et; col < 4 * Z; col += NT) {
       const int p4 = col / Z, jj = col % Z;
       const float t = scs[col];
-      if (t != 0.f && (p4 < 2 || prm.prior_mode == 2)) atomicAdd((p4 < 2 ? prm.db_enc : prm.db_prior) + (p4 & 1) * Z + jj, t);
+      if (prm.db_enc && t != 0.f && (p4 < 2 || prm.prior_mode == 2)) atomicAdd((p4 < 2 ? prm.db_enc : prm.db_prior) + (p4 & 1) * Z + jj, t);
     }
     asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
   }

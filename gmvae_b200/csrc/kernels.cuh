@@ -725,11 +725,13 @@ __global__ void dist_row_kernel(int op, const float* __restrict__ a, const float
 // ---- VAE_GMP mixture prior (vae.py:231-244, 181): forward value and every gradient -------------
 // log p(z) = logsumexp_k [ log_softmax(m)_k + log N(z; loc_k, softplus(raw_scale_k)) ]
 // One warp per row; lanes stride over Z.  Adds -log p / B to the KL accumulator, writes
-// d kl/dz (prior part) to dz_prior, and accumulates d loc, d raw_scale_diag, d mixture_logits.
+// d kl/dz (prior part) to dz_prior, and accumulates d loc, d raw_scale_diag, d mixture_logits (deterministic mode: into the
+// fixed-point sums fx = [K mixture logits | K*Z loc | K*Z raw_scale_diag] instead).
 __global__ void gmp_prior_kernel(const float* __restrict__ z, const float* __restrict__ loc,
                                  const float* __restrict__ raw_scale, const float* __restrict__ mix_logits, int B, int K,
                                  int Z, float inv_bg, float* __restrict__ dz_prior, float* __restrict__ d_loc,
-                                 float* __restrict__ d_raw_scale, float* __restrict__ d_mix, float* __restrict__ acc) {
+                                 float* __restrict__ d_raw_scale, float* __restrict__ d_mix, float* __restrict__ acc,
+                                 unsigned long long* __restrict__ fx) {
   griddep_wait();
   griddep_launch();
   extern __shared__ float sm[];  // per warp: K log-weights
@@ -768,16 +770,24 @@ __global__ void gmp_prior_kernel(const float* __restrict__ z, const float* __res
     for (int j = lane; j < Z; j += 32) dz_prior[(int64_t)row * Z + j] = 0.f;
     for (int k = 0; k < K; ++k) {
       const float r = expf(lw[k] - logp);  // responsibility
-      if (lane == 0) atomicAdd(d_mix + k, -(r - expf(mix_logits[k] - mlse)) * inv_bg);
+      if (lane == 0) {
+        const float g = -(r - expf(mix_logits[k] - mlse)) * inv_bg;
+        if (fx) fx_add(fx, k, g); else atomicAdd(d_mix + k, g);
+      }
       for (int j = lane; j < Z; j += 32) {
         float raw = raw_scale[k * Z + j];
         float sc = softplus_f(raw);
         float d = z[(int64_t)row * Z + j] - loc[k * Z + j];
         float is2 = 1.f / (sc * sc);
         dz_prior[(int64_t)row * Z + j] += r * d * is2 * inv_bg;
-        atomicAdd(d_loc + k * Z + j, -r * d * is2 * inv_bg);
         float dsc = -r * (d * d * is2 / sc - 1.f / sc) * inv_bg;
-        atomicAdd(d_raw_scale + k * Z + j, dsc * sigmoid_f(raw));
+        if (fx) {
+          fx_add(fx, K + k * Z + j, -r * d * is2 * inv_bg);
+          fx_add(fx, K + K * Z + k * Z + j, dsc * sigmoid_f(raw));
+        } else {
+          atomicAdd(d_loc + k * Z + j, -r * d * is2 * inv_bg);
+          atomicAdd(d_raw_scale + k * Z + j, dsc * sigmoid_f(raw));
+        }
       }
     }
   }
@@ -1025,8 +1035,11 @@ __global__ void head_y_m_bwd_kernel(const float* __restrict__ logits, const floa
 // ---- bias gradients: db[n] += sum_m dY[m,n] -----------------------------------------------------
 // Each thread owns 8 consecutive columns (one 16-byte load per row for bf16); a block covers
 // 256 columns x `rows_per_block` rows with 8 row-lanes, reduced through shared memory.
+// part != null (deterministic mode): row block y stores its sums to part[y * N + n] (every column, zeros too) instead of adding
+// them to db; det_reduce_kernel adds the row blocks in order.
 template <typename T>
-__global__ void colsum_kernel(const T* __restrict__ dY, int64_t ld, int M, int N, int rows_per_block, float* __restrict__ db) {
+__global__ void colsum_kernel(const T* __restrict__ dY, int64_t ld, int M, int N, int rows_per_block, float* __restrict__ db,
+                              float* __restrict__ part) {
   griddep_wait();
   griddep_launch();
   __shared__ float sm[8][32][9];
@@ -1055,7 +1068,35 @@ __global__ void colsum_kernel(const T* __restrict__ dY, int64_t ld, int M, int N
 #pragma unroll
   for (int i = 0; i < 8; ++i) t += sm[i][cx][cj];
   const int n = blockIdx.x * 256 + c;
+  if (part) { if (n < N) part[(int64_t)blockIdx.y * N + n] = t; return; }
   if (n < N && t != 0.f) atomicAdd(db + n, t);
+}
+
+// ---- deterministic mode: the reduction step ------------------------------------------------------
+// One launch after the step's last GEMM, before the gradient exchange.  Segment blockIdx.y is a rows x cols block of the gradient
+// buffer, element (r, c) at dst[r * ld_dst + c]:
+//   part != null: part[0 * part_stride + r * ld_part + c] + part[1 * part_stride + ...] + ...  (nparts partials: the k-splits of a
+//                 weight gradient, chain_sched.cuh det_slice_index, or the row blocks of a column sum -- added in index order)
+//   fx != null:   the fixed-point sum r * cols + c (common.cuh fx_add), NaN if it was flagged
+constexpr int DET_MAX_SEGS = 64;
+struct DetSeg { float* dst; const float* part; const unsigned long long* fx; long long part_stride; int rows, cols, nparts, ld_dst, ld_part, pad; };
+struct DetSegs { int nseg; DetSeg s[DET_MAX_SEGS]; };
+__global__ void det_reduce_kernel(const __grid_constant__ DetSegs segs) {
+  griddep_wait();
+  griddep_launch();
+  const DetSeg& g = segs.s[blockIdx.y];
+  const long long n = (long long)g.rows * g.cols;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int r = (int)(i / g.cols), c = (int)(i % g.cols);
+    float v = 0.f;
+    if (g.fx) {
+      v = g.fx[2 * i + 1] ? __int_as_float(0x7fffffff) : (float)((double)(long long)g.fx[2 * i] * (1.0 / (double)(1ull << FX_SHIFT)));
+    } else {
+      const float* p = g.part + (long long)r * g.ld_part + c;
+      for (int s = 0; s < g.nparts; ++s) v += p[(long long)s * g.part_stride];
+    }
+    g.dst[(long long)r * g.ld_dst + c] = v;
+  }
 }
 
 // ---- loss terms ---------------------------------------------------------------------------------

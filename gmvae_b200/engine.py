@@ -26,7 +26,8 @@ class Engine:
                  sigma_min: float = 0.0, raw_sigma_bias: float = 0.5, gen_bias_init: float = 0.0,
                  temperature: float = 1.0, learning_rate: float = 1e-3, beta1: float = 0.9,
                  beta2: float = 0.999, epsilon: float = 1e-8, device: Optional[int] = None,
-                 seed: Optional[int] = None, init: bool = True):
+                 seed: Optional[int] = None, init: bool = True, deterministic: bool = False):
+        """deterministic=True: bitwise-reproducible training steps (gmvae_config::deterministic, DESIGN.md section 9)."""
         if not torch.cuda.is_available():
             raise RuntimeError("gmvae_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = _lib.load()
@@ -37,6 +38,7 @@ class Engine:
         self.hidden_sizes = [int(h) for h in hidden_sizes]
         self.mixture_components = int(mixture_components)
         self.max_batch = int(max_batch)
+        self.deterministic = bool(deterministic)
         cfg = _lib.Config()
         cfg.abi_version = _lib.ABI_VERSION
         cfg.model = _lib.MODEL_IDS[model]
@@ -54,6 +56,7 @@ class Engine:
         cfg.gen_bias_init, cfg.temperature = gen_bias_init, temperature
         cfg.learning_rate, cfg.beta1, cfg.beta2, cfg.epsilon = learning_rate, beta1, beta2, epsilon
         cfg.device = self.device_index
+        cfg.deterministic = 1 if self.deterministic else 0
         self.cfg = cfg
         self._h = C.c_void_p()
         _lib.check(self.lib.gmvae_create(C.byref(cfg), C.byref(self._h)), "gmvae_create")
@@ -346,6 +349,10 @@ class Engine:
         import os
         if os.environ.get("GMVAE_DP_PEER", "1") != "0":
             self.attach_peers()
+        if self.deterministic and not self.peer_attached:
+            import warnings
+            warnings.warn("deterministic=True: the NCCL all-reduce adds the ranks' gradients in an order of its own; "
+                          "steps are bitwise reproducible only with the peer-memory exchange")
 
     def attach_peers(self) -> bool:
         """The exchange step over NVLink peer memory, fused with Adam (csrc/peer.cuh), in place of the NCCL all-reduce (default

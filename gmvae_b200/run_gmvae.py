@@ -1,6 +1,6 @@
 """Command line -- same flags, defaults and `--flag=value` syntax as
 /root/reference/scripts/run_gmvae.py:11-58 (tf.app.flags), plus additive flags (`--precision`,
-`--objective`, `--dataset_path`, `--image_summaries`).  Data parallelism needs no flag: launch with
+`--objective`, `--dataset_path`, `--image_summaries`, `--deterministic`).  Data parallelism needs no flag: launch with
 `torchrun --nproc-per-node N -m gmvae_b200.run_gmvae ...` and `--batch_size` is the per-GPU batch.
 
     python -m gmvae_b200.run_gmvae --mode=train --model=gmvae --latent_size=64 --hidden_size=512 \
@@ -44,6 +44,8 @@ def build_parser() -> argparse.ArgumentParser:
                    "default $GMVAE_MNIST_DIR, else a synthetic stand-in (the reference downloads through TFDS).")
     p.add_argument("--image_summaries", type=int, default=1, help="Write the input / reconstruction / sample tiles with "
                    "every summary (the reference always does).")
+    p.add_argument("--deterministic", action="store_true", help="Bitwise-reproducible training steps: the same seed, data and "
+                   "configuration give identical parameters (slower; DESIGN.md section 9).")
     return p
 
 

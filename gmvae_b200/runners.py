@@ -102,7 +102,8 @@ def logdir_for(config) -> str:
 
 def _configure(model, config, device: int):
     model.configure(precision=getattr(config, "precision", "bf16"), objective=getattr(config, "objective", "reference"),
-                    learning_rate=getattr(config, "learning_rate", 1e-3), max_batch=config.batch_size, device=device)
+                    learning_rate=getattr(config, "learning_rate", 1e-3), max_batch=config.batch_size, device=device,
+                    deterministic=getattr(config, "deterministic", False))
     model.random_seed = config.random_seed
     return model.engine(config.batch_size)
 

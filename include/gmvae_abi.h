@@ -69,7 +69,12 @@ typedef struct gmvae_config {
   float learning_rate;        /* --learning_rate; tf.train.AdamOptimizer defaults below */
   float beta1, beta2, epsilon;
   int32_t device;             /* CUDA ordinal */
-  int32_t reserved[7];
+  /* 1: bitwise-reproducible training steps.  Two steps with the same build, device type, configuration, parameters, Adam state,
+   * global step, seed and inputs give identical gradients, loss terms, parameters and Adam moments (eager or graph, one GPU or
+   * the peer-memory exchange; not the NCCL all-reduce).  Sums whose addends arrive in no fixed order are taken in a fixed order
+   * or in integer fixed point; costs step time (DESIGN.md section 9).  objective=reference only; 0 (default): the fastest plan. */
+  int32_t deterministic;
+  int32_t reserved[6];
 } gmvae_config;
 
 /* One trainable variable of the flat parameter buffer.  Names are the reference's TF
