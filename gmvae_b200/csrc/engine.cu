@@ -7,6 +7,7 @@
 #include <nccl.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -936,7 +937,7 @@ static int bias_grad(gmvae_handle* h, const T* dY, int64_t ldy, int M, int N, fl
 
 // ============================================================================ MLP passes
 // Every GEMM-operand activation buffer has its row stride rounded up to 8 elements (16 bytes, the
-// TMA requirement); the padding columns are never written and stay zero from allocation.
+// TMA requirement); the padding columns are never written and stay zero from gmvae_bind, which clears the workspace.
 static inline int ldp(int n) { return round_up(n, 8); }
 
 template <typename A> struct MlpBufs { std::vector<A*> hid, dhid; std::vector<uint32_t*> bits; };
@@ -1575,8 +1576,7 @@ static int forward_backward_marginal(gmvae_handle* h, const uint8_t* x_u8, int B
     const int nb = std::min(h->chunk_samples, B - b0), R = nb * K, row0 = b0 * K;
     // h1 for all components of the chunk
     {
-      const int64_t work = (int64_t)R * (H0 / 4);
-      GM_REQUIRE(H0 % 4 == 0, "objective=marginal needs hidden sizes that are multiples of 4");
+      const int64_t work = (int64_t)R * (H0 / 4);                  // H0 % 4 == 0: checked by gmvae_create
       const int blocks = (int)std::min<int64_t>((work + 255) / 256, 16 * tc::num_sms());
       GM_CHECK_CUDA(launch_k(expand_h1_kernel<A>, dim3(blocks), dim3(256), 0, st, true, (const float*)(xproj + (int64_t)b0 * H0), (int64_t)H0, Wy,
                              (const float*)(h->params + enc_l0.b_off), R, K, H0, enc.hid[0], (int64_t)H0p));
@@ -1611,8 +1611,7 @@ static int forward_backward_marginal(gmvae_handle* h, const uint8_t* x_u8, int B
     {
       const int lanes = 256 / Z;
       const int blocks = std::max(1, std::min(2 * tc::num_sms(), (R + lanes - 1) / lanes));
-      const size_t smem = (size_t)(2 * 256 + K * 2 * Z) * sizeof(float);
-      GM_REQUIRE(smem <= 200 * 1024, "objective=marginal: mixture_components * latent_size too large for the prior-table gradient tile");
+      const size_t smem = (size_t)(2 * 256 + K * 2 * Z) * sizeof(float);   // <= 200 KB: checked by gmvae_create
       static size_t smem_set_by_dev[64] = {};
       size_t& smem_set = smem_set_by_dev[tc::current_device()];
       if (smem > smem_set) {
@@ -1705,8 +1704,13 @@ int gmvae_create(const gmvae_config* cfg, gmvae_handle** out) {
   if (cfg->model != GMVAE_MODEL_VAE)
     GM_REQUIRE(cfg->mixture_components >= 1 && cfg->mixture_components <= HEAD_MAXK, "mixture_components must be in [1,128]");
   GM_REQUIRE(cfg->objective == GMVAE_OBJECTIVE_REFERENCE || cfg->model == GMVAE_MODEL_GMVAE, "objective applies to GMVAE only");
-  if (cfg->objective == GMVAE_OBJECTIVE_MARGINAL)
+  if (cfg->objective == GMVAE_OBJECTIVE_MARGINAL) {
     GM_REQUIRE(cfg->num_hidden >= 1 && cfg->latent_size <= 256, "objective=marginal needs at least one hidden layer and latent_size <= 256");
+    // expand_h1_kernel reads layer 0 in float4 groups; head_z_m_bwd_kernel holds the K x 2Z prior-table gradient in shared memory
+    GM_REQUIRE(cfg->hidden_sizes[0] % 4 == 0, "objective=marginal needs hidden sizes that are multiples of 4");
+    GM_REQUIRE((2 * 256 + (int64_t)cfg->mixture_components * 2 * cfg->latent_size) * (int64_t)sizeof(float) <= 200 * 1024,
+               "objective=marginal: mixture_components * latent_size too large for the prior-table gradient tile");
+  }
   GM_REQUIRE(cfg->deterministic == 0 || cfg->deterministic == 1, "deterministic must be 0 or 1");
   if (cfg->deterministic) {
     GM_REQUIRE(cfg->objective == GMVAE_OBJECTIVE_REFERENCE, "deterministic mode supports objective=reference only");
@@ -1716,6 +1720,15 @@ int gmvae_create(const gmvae_config* cfg, gmvae_handle** out) {
       GM_REQUIRE(!e || atoi(e) == 0, std::string("deterministic mode cannot be combined with ") + v);
     }
   }
+  // hyperparameters: a non-finite or out-of-range value would only show up as NaN (or inf) in the first step
+  GM_REQUIRE(std::isfinite(cfg->temperature) && cfg->temperature > 0.f, "temperature must be finite and > 0");
+  GM_REQUIRE(std::isfinite(cfg->sigma_min) && cfg->sigma_min >= 0.f, "sigma_min must be finite and >= 0");
+  GM_REQUIRE(std::isfinite(cfg->raw_sigma_bias), "raw_sigma_bias must be finite");
+  GM_REQUIRE(std::isfinite(cfg->gen_bias_init), "gen_bias_init must be finite");
+  GM_REQUIRE(std::isfinite(cfg->learning_rate) && cfg->learning_rate > 0.f, "learning_rate must be finite and > 0");
+  GM_REQUIRE(cfg->beta1 >= 0.f && cfg->beta1 < 1.f, "beta1 must be in [0, 1)");
+  GM_REQUIRE(cfg->beta2 >= 0.f && cfg->beta2 < 1.f, "beta2 must be in [0, 1)");
+  GM_REQUIRE(std::isfinite(cfg->epsilon) && cfg->epsilon >= 0.f, "epsilon must be finite and >= 0");
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0) {
@@ -1779,6 +1792,10 @@ int gmvae_bind(gmvae_handle* h, float* params, float* grads, float* adam_m, floa
   GM_REQUIRE(!h->peer_ready, "gmvae_bind after gmvae_peer_attach is not supported");
   h->params = params; h->grads = grads; h->grads_bound = grads; h->adam_m = adam_m; h->adam_v = adam_v;
   h->ws = reinterpret_cast<uint8_t*>(workspace); h->ws_bytes = workspace_bytes;
+  // The padding columns of the activation buffers are never written and the tensor-core GEMMs contract over them (kpad): they
+  // must hold zeros, not whatever the caller's allocation held (0 x NaN is NaN).  Once here, outside the step.
+  GM_CHECK_CUDA(cudaMemsetAsync(workspace, 0, h->ws_needed, 0));
+  GM_CHECK_CUDA(cudaStreamSynchronize(0));
   h->shadow_host.clear(); h->shadow_tiles = 0;
   if (h->bf16_mode()) {
     Mlp* mlps[4] = {&h->decoder, &h->encoder, &h->encoder_y, &h->prior_gmm};

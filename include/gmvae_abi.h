@@ -99,7 +99,9 @@ GMVAE_API int gmvae_num_params(const gmvae_handle* h);
 GMVAE_API int gmvae_param_table(const gmvae_handle* h, gmvae_param_desc* out, int cap);
 
 GMVAE_API size_t gmvae_workspace_bytes(const gmvae_handle* h);
-/* params/adam_m/adam_v: float[param_count]; grads: float[grad_count]; workspace: bytes above. */
+/* params/adam_m/adam_v: float[param_count]; grads: float[grad_count]; workspace: bytes above, 256-byte aligned, any contents:
+ * gmvae_bind clears it (synchronously, on the legacy default stream) before it returns, bf16 weight copies included, so
+ * gmvae_params_updated follows a bind. */
 GMVAE_API int gmvae_bind(gmvae_handle* h, float* params, float* grads, float* adam_m, float* adam_v,
                void* workspace, size_t workspace_bytes);
 /* Call after writing `params` from outside (initialisation, checkpoint restore): refreshes

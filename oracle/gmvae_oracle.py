@@ -183,7 +183,8 @@ def loss_terms(spec: Spec, params: Dict[str, torch.Tensor], x: torch.Tensor,
                eps: torch.Tensor, u: Optional[torch.Tensor] = None,
                objective: str = "reference", global_batch: Optional[int] = None, q: Exact = EXACT) -> Dict[str, torch.Tensor]:
     """Forward pass.  Returns loss, nll, kl_div_z, nent (nent == 0 for VAE models) and a few
-    intermediates used by the tests.  `global_batch` (default: len(x)) is the divisor of the
+    intermediates used by the tests (among them the clamped scales sigma_q of q(z|.) and, for the
+    GMVAE, sigma_p of p(z|y)).  `global_batch` (default: len(x)) is the divisor of the
     batch means, so that shards of a data-parallel batch can be summed."""
     dt = next(iter(params.values())).dtype
     x = x.to(dt)
@@ -204,7 +205,7 @@ def loss_terms(spec: Spec, params: Dict[str, torch.Tensor], x: torch.Tensor,
             logp = torch.logsumexp(comp + torch.log_softmax(params["mixture_logits"], -1)[None], dim=-1)
         kl = (logq - logp).sum() / Bg
         zero = torch.zeros((), dtype=dt)
-        out.update(loss=nll + kl, nll=nll, kl_div_z=kl, nent=zero, z=z, logits_x=logits)
+        out.update(loss=nll + kl, nll=nll, kl_div_z=kl, nent=zero, z=z, logits_x=logits, sigma_q=sg_q)
         return out
     if spec.model != "gmvae":
         raise ValueError(spec.model)
@@ -220,7 +221,7 @@ def loss_terms(spec: Spec, params: Dict[str, torch.Tensor], x: torch.Tensor,
         logits = q.grad(mlp(params, "decoder", q.fwd(z), L, q)) + spec.gen_bias_init   # gmvae.py:251
         nll = -bernoulli_log_prob(x, logits).sum() / Bg                    # gmvae.py:254
         kl = (mvn_diag_log_prob(z, mu_q, sg_q) - mvn_diag_log_prob(z, mu_p, sg_p)).sum() / Bg  # :258
-        out.update(y=y, z=z, logits_x=logits)
+        out.update(y=y, z=z, logits_x=logits, sigma_q=sg_q, sigma_p=sg_p)
     elif objective == "marginal":
         # SURVEY.md Appendix A.3: the reference's own blocks evaluated at y = e_k for every k,
         # weighted by q(y|x), with the analytic Gaussian KL.  eps has shape [B, K, Z].
@@ -248,7 +249,7 @@ def loss_terms(spec: Spec, params: Dict[str, torch.Tensor], x: torch.Tensor,
         klk = (torch.log(sg_p[None] / sg_q) + (sg_q ** 2 + (mu_q - mu_p[None]) ** 2) / (2 * sg_p[None] ** 2) - 0.5).sum(-1)
         nll = -(py * rec).sum() / Bg
         kl = (py * klk).sum() / Bg
-        out.update(z=z, logits_x=logits)
+        out.update(z=z, logits_x=logits, sigma_q=sg_q, sigma_p=sg_p)
     else:
         raise ValueError(objective)
     out.update(loss=nll + kl + nent, nll=nll, kl_div_z=kl, nent=nent, logits_y=ly)

@@ -22,19 +22,54 @@ CONFIGS = {
     # 16 < K <= 32, nothing a multiple of a tile, more than one 128-row block
     "k20_ragged": dict(model="gmvae", latent_size=40, hidden_sizes=[96, 72], mixture_components=20, batch=150, data_size=200),
     "k17_gmp": dict(model="vae_gmp", latent_size=20, hidden_sizes=[64], mixture_components=17, batch=130, data_size=96),
+    # the dispatch boundaries of the heads (engine.cu forward_encoder / the z head) and padded row strides
+    # K = 1: a one-way softmax (y = 1, zero entropy, exactly zero encoder_y gradients)
+    "k1_gmvae": dict(model="gmvae", latent_size=16, hidden_sizes=[64], mixture_components=1, batch=40, data_size=120),
+    # K = 16: the largest y head fused into the GEMM epilogue (Kp = 16, the second uint4 store)
+    "k16_gmvae": dict(model="gmvae", latent_size=24, hidden_sizes=[64, 48], mixture_components=16, batch=100, data_size=200),
+    # K = 32 / 33: the last lane slot of the warp head that is full / the first one past it
+    "k32_gmvae": dict(model="gmvae", latent_size=16, hidden_sizes=[80], mixture_components=32, batch=90, data_size=144),
+    "k33_gmvae": dict(model="gmvae", latent_size=16, hidden_sizes=[80], mixture_components=33, batch=90, data_size=144),
+    # K = 128 = HEAD_MAXK; VAE_GMP with a small Z: gmp_prior_kernel's shared-memory table
+    "k128_gmvae": dict(model="gmvae", latent_size=32, hidden_sizes=[96], mixture_components=128, batch=150, data_size=200),
+    "k128_gmp": dict(model="vae_gmp", latent_size=4, hidden_sizes=[64], mixture_components=128, batch=100, data_size=120),
+    # Z = 1, 3: the _cs z head with Zp = 8
+    "z1_vae": dict(model="vae", latent_size=1, hidden_sizes=[48], mixture_components=1, batch=60, data_size=112),
+    "z3_gmvae": dict(model="gmvae", latent_size=3, hidden_sizes=[40], mixture_components=5, batch=70, data_size=96),
+    # Z = 65: odd width past 64 (generic forward head, _cs backward with 3 rows per block)
+    "z65_gmp": dict(model="vae_gmp", latent_size=65, hidden_sizes=[64], mixture_components=6, batch=80, data_size=128),
+    # Z = 256: the largest v4 / _cs head; Z = 260: the generic z head with the bias gradient left unfused
+    "z256_gmvae": dict(model="gmvae", latent_size=256, hidden_sizes=[128], mixture_components=4, batch=60, data_size=160),
+    "z260_gmvae": dict(model="gmvae", latent_size=260, hidden_sizes=[96], mixture_components=3, batch=40, data_size=120),
+    "z260_vae": dict(model="vae", latent_size=260, hidden_sizes=[128], mixture_components=1, batch=50, data_size=104),
+    # hidden widths that are not multiples of 8: padded row strides that the tensor-core GEMMs contract over
+    "h33_7": dict(model="gmvae", latent_size=12, hidden_sizes=[33, 7], mixture_components=6, batch=64, data_size=120),
+    "h129_gmp": dict(model="vae_gmp", latent_size=20, hidden_sizes=[129], mixture_components=5, batch=50, data_size=152),
+    # odd image rows: the byte path of the BCE x load
+    "d97": dict(model="gmvae", latent_size=10, hidden_sizes=[40], mixture_components=5, batch=80, data_size=97),
+    # objective M shapes (its layer 0 must be a multiple of 4 wide), also run under objective R
+    "m_h36_20_k33": dict(model="gmvae", latent_size=12, hidden_sizes=[36, 20], mixture_components=33, batch=20, data_size=100),
+    "m_k128_z8": dict(model="gmvae", latent_size=8, hidden_sizes=[32], mixture_components=128, batch=10, data_size=64),
 }
+
+
+# Model hyperparameters a cfg dict may set; absent ones take the defaults of runners.create_model (the oracle's Spec and Engine
+# share them: sigma_min 0, raw_sigma_bias 0.5, gen_bias_init 0, temperature 1).
+KNOBS = ("sigma_min", "raw_sigma_bias", "gen_bias_init", "temperature")
 
 
 def make_spec(cfg):
     return O.Spec(model=cfg["model"], data_size=cfg.get("data_size", 784), latent_size=cfg["latent_size"],
-                  hidden_sizes=list(cfg["hidden_sizes"]), mixture_components=cfg["mixture_components"])
+                  hidden_sizes=list(cfg["hidden_sizes"]), mixture_components=cfg["mixture_components"],
+                  **{k: cfg[k] for k in KNOBS if k in cfg})
 
 
 def make_engine(cfg, precision, max_batch=None, objective="reference", **kw):
     import gmvae_b200
     return gmvae_b200.Engine(model=cfg["model"], data_size=cfg.get("data_size", 784), latent_size=cfg["latent_size"],
                              hidden_sizes=cfg["hidden_sizes"], mixture_components=cfg["mixture_components"],
-                             precision=precision, objective=objective, max_batch=max_batch or cfg["batch"], init=False, **kw)
+                             precision=precision, objective=objective, max_batch=max_batch or cfg["batch"], init=False,
+                             **{k: cfg[k] for k in KNOBS if k in cfg}, **kw)
 
 
 def perturbed_params(spec, seed=2024, bias_scale=0.05):
@@ -162,3 +197,30 @@ class Bf16Model(O.Exact):
 
     def yin(self, t):            # y is the bf16 operand of the second K segment (tensor-core path)
         return _RoundFwd.apply(t) if self.tcw else t
+
+
+# --------------------------------------------------------------------------- sigma_min cases
+def active_clamp(cfg, params, x, eps, u=None, objective="reference"):
+    """`cfg` with raw_sigma_bias = 0 and a sigma_min that clamps about half of the scales: the midpoint of the widest gap between
+    consecutive values of softplus(raw) (q(z) and, for the GMVAE, p(z|y) pooled) between their 40th and 60th percentiles, on
+    these weights and inputs, rounded to fp32 (the type of gmvae_config::sigma_min).  Taking a gap keeps every entry off the
+    kink of the clamp."""
+    t = O.loss_terms(make_spec(dict(cfg, sigma_min=0.0, raw_sigma_bias=0.0)), params, x, eps, u, objective)
+    s = torch.cat([t[k].reshape(-1) for k in ("sigma_q", "sigma_p") if k in t]).sort().values
+    lo, hi = int(0.4 * s.numel()), int(0.6 * s.numel())
+    i = lo + int((s[lo + 1:hi + 1] - s[lo:hi]).argmax())
+    thr = torch.tensor(0.5 * (s[i] + s[i + 1]).item(), dtype=torch.float32).item()
+    return dict(cfg, sigma_min=thr, raw_sigma_bias=0.0)
+
+
+def clamp_stats(cfg, params, x, eps, u=None, objective="reference"):
+    """From the oracle's forward pass: the share of the scales of q(z) and p(z|y) that cfg's sigma_min clamps, and how many
+    entries of softplus(raw + raw_sigma_bias) lie within 1e-5 (relative) of it."""
+    t = O.loss_terms(make_spec(dict(cfg, sigma_min=0.0)), params, x, eps, u, objective)
+    thr = float(cfg.get("sigma_min", 0.0))
+    out = {"sigma_min": thr, "near_threshold": 0}
+    for k in ("sigma_q", "sigma_p"):
+        if k in t:
+            out[k + "_clamped"] = (t[k] < thr).double().mean().item()
+            out["near_threshold"] += int(((t[k] - thr).abs() <= 1e-5 * thr).sum())
+    return out

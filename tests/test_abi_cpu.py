@@ -44,6 +44,7 @@ def test_no_cpu_fallback():
     cfg = _lib.Config()
     cfg.abi_version = 1; cfg.model = 2; cfg.precision = 1; cfg.data_size = 784; cfg.latent_size = 8
     cfg.mixture_components = 10; cfg.num_hidden = 1; cfg.hidden_sizes[0] = 64; cfg.max_batch = 16
+    cfg.raw_sigma_bias = 0.5; cfg.temperature = 1.0; cfg.learning_rate = 1e-3; cfg.beta1 = 0.9; cfg.beta2 = 0.999; cfg.epsilon = 1e-8
     h = C.c_void_p()
     rc = lib.gmvae_create(C.byref(cfg), C.byref(h))
     assert rc != 0 and b"no CPU fallback" in lib.gmvae_last_error()

@@ -24,6 +24,10 @@ CASES = {
     "cfg4": dict(model="gmvae", latent_size=64, hidden_sizes=[512, 512], mixture_components=10, batch=16384),
     "cfg5_model": dict(model="gmvae", latent_size=128, hidden_sizes=[1024, 1024], mixture_components=50, batch=8192),
     "k17": dict(model="gmvae", latent_size=40, hidden_sizes=[96, 72], mixture_components=17, batch=150, data_size=200),
+    # widths that are not multiples of 4 (det_slice_ld, colsum_kernel), the generic z head, the largest K
+    "odd": dict(model="gmvae", latent_size=3, hidden_sizes=[33, 7], mixture_components=5, batch=300, data_size=97),
+    "z260": dict(model="vae_gmp", latent_size=260, hidden_sizes=[130], mixture_components=3, batch=200, data_size=120),
+    "k128": dict(model="gmvae", latent_size=20, hidden_sizes=[90], mixture_components=128, batch=260, data_size=150),
 }
 PARAMS = [(n, "bf16") for n in CASES] + [(n, "fp32") for n in ("vae", "vae_gmp", "gmvae")]
 

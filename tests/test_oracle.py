@@ -150,15 +150,29 @@ def test_against_torch_distributions(model):
         assert abs(a.item() - b.item()) <= 1e-10 * max(1.0, abs(b.item()))
 
 
-@pytest.mark.parametrize("model,objective", [("vae", "reference"), ("vae_gmp", "reference"),
-                                             ("gmvae", "reference"), ("gmvae", "marginal")])
-def test_finite_differences(model, objective):
-    spec = O.Spec(model, data_size=20, latent_size=4, hidden_sizes=[6, 5], mixture_components=3)
+# a non-default set of every model hyperparameter; sigma_min clamps part of the scales, none of them within 1e-3 of the kink
+KNOBS_FD = dict(temperature=0.7, sigma_min=0.55, raw_sigma_bias=-0.2, gen_bias_init=-0.8)
+FD_CASES = [pytest.param(m, o, {}, id=f"{m}-{o}") for m, o in (("vae", "reference"), ("vae_gmp", "reference"), ("gmvae", "reference"),
+                                                              ("gmvae", "marginal"))]
+FD_CASES += [pytest.param(m, o, KNOBS_FD, id=f"{m}-{o}-knobs") for m, o in (("vae_gmp", "reference"), ("gmvae", "reference"),
+                                                                             ("gmvae", "marginal"))]
+
+
+@pytest.mark.parametrize("model,objective,knobs", FD_CASES)
+def test_finite_differences(model, objective, knobs):
+    spec = O.Spec(model, data_size=20, latent_size=4, hidden_sizes=[6, 5], mixture_components=3, **knobs)
     params = O.init_params(spec, seed=5)
     for n in params:
         if n.endswith("/b"):
             params[n] = 0.2 * torch.randn(params[n].shape, dtype=F64, generator=torch.Generator().manual_seed(len(n)))
     x, _, eps, u = O.synthetic_batch(spec, 6, objective=objective)
+    if knobs:
+        # the clamp is active and every scale is away from its kink, where the loss is not differentiable
+        t = O.loss_terms(O.Spec(model, data_size=20, latent_size=4, hidden_sizes=[6, 5], mixture_components=3,
+                                **dict(knobs, sigma_min=0.0)), params, x, eps, u, objective)
+        s = torch.cat([t[k].reshape(-1) for k in ("sigma_q", "sigma_p") if k in t])
+        assert 0.1 < (s < spec.sigma_min).double().mean().item() < 0.9
+        assert (s - spec.sigma_min).abs().min().item() > 1e-3
     _, grads = O.loss_and_grads(spec, params, x, eps, u, objective)
     g = torch.Generator().manual_seed(9)
     h = 1e-6
@@ -217,3 +231,57 @@ def test_bf16_rounding_model_explains_gradient_gap():
     assert abs(t0["loss"].item() - t1["loss"].item()) / t0["loss"].item() < 2e-3
     worst = max(((g1[n] - g0[n]).norm() / g0[n].norm()).item() for n in g0)
     assert 1e-3 < worst < 0.1
+
+
+# --------------------------------------------------------------------------- hyperparameter sensitivity
+def _knob_cases():
+    """The hyperparameter cases of tests/test_config_edges_gpu.py on their small shapes: (id, cfg, objective, knob values)."""
+    from tests.helpers import CONFIGS
+    out = []
+    for name in ("cfg3", "k20_ragged"):
+        for T in (0.5, 2.0):
+            out.append((f"{name}-T={T}", CONFIGS[name], "reference", dict(temperature=T)))
+    for name, obj in (("cfg1", "reference"), ("tiny_gmp", "reference"), ("cfg3", "reference"), ("tiny_gmvae", "marginal")):
+        out.append((f"{name}-{obj}-gen_bias_init", CONFIGS[name], obj, dict(gen_bias_init=-1.5)))
+        for knobs in ("dropin", "active"):
+            out.append((f"{name}-{obj}-sigma={knobs}", CONFIGS[name], obj, knobs))
+    return out
+
+
+KNOB_CASES = _knob_cases()
+FP32_BAR = 1e-5          # what the GPU tests hold the fp32 validation mode to, per loss term and per gradient tensor
+
+
+# the tensors each knob acts on first: the networks whose output it enters
+DIRECT = {"temperature": ("encoder_y_fcnet/",), "gen_bias_init": ("decoder_fcnet/",),
+          "sigma": ("encoder_fcnet/", "encoder_gmm_fcnet/", "prior_gmm_fcnet/")}
+
+
+@pytest.mark.parametrize("case", KNOB_CASES, ids=[c[0] for c in KNOB_CASES])
+def test_knob_values_move_the_oracle(case):
+    """The oracle at each knob value of the GPU tests and at the default differs by at least 20 x the fp32 bar in the loss and in
+    every gradient tensor of the networks the knob acts on (a kernel that ignored the knob fails there), and by at least 10 x the
+    bar in every other tensor it reaches (one equal to 1e-12 is not reached, e.g. the prior's gradients by gen_bias_init).  Loss
+    terms other than the loss are not held: the relaxed sample reaches nll through z only, and T = 0.5 moves it by 2e-6 on cfg3."""
+    from tests.helpers import active_clamp, make_spec, perturbed_params
+    cid, cfg, obj, knobs = case
+    spec0 = make_spec(cfg)
+    params = perturbed_params(spec0)
+    x, _, eps, u = O.synthetic_batch(spec0, cfg["batch"], objective=obj)
+    if knobs == "dropin":
+        knobs = dict(sigma_min=0.001, raw_sigma_bias=0.25)
+    elif knobs == "active":
+        knobs = {k: v for k, v in active_clamp(cfg, params, x, eps, u, obj).items() if k in ("sigma_min", "raw_sigma_bias")}
+    direct = DIRECT["sigma" if "sigma_min" in knobs else next(iter(knobs))]
+    t0, g0 = O.loss_and_grads(spec0, params, x, eps, u, obj)
+    t1, g1 = O.loss_and_grads(make_spec(dict(cfg, **knobs)), params, x, eps, u, obj)
+    assert abs(t1["loss"].item() - t0["loss"].item()) / abs(t0["loss"].item()) > 20 * FP32_BAR
+    n_direct = 0
+    for n in g0:
+        d = ((g1[n] - g0[n]).norm() / g0[n].norm().clamp_min(1e-30)).item()
+        if n.startswith(direct):
+            n_direct += 1
+            assert d > 20 * FP32_BAR, (cid, n, d)
+        else:
+            assert d < 1e-12 or d > 10 * FP32_BAR, (cid, n, d)
+    assert n_direct >= 2

@@ -37,6 +37,17 @@ MODEL_TENSOR_BOUND = {"cfg5_small": 1.2e-2}
 # fp32 arithmetic itself is the limit: the CPU oracle evaluated in fp32 differs from the fp64 oracle by 4.0e-5 on
 # decoder linear_0/w (measured in this repo, same inputs); the CUDA fp32 mode measures 2.7e-5.
 FP32_TOL = {("cfg5_small", "marginal"): 1e-4}
+# bf16 loss terms: h33_7 (a 7-wide hidden layer, Z = 12) -- the oracle under the bf16 rounding model moves kl_div_z (1.82 nats) by
+# 3.99e-3 nats = 2.19e-3 relative from the exact oracle; the CUDA path measures 2.19e-3 (B200).
+TERMS_BF16_TOL = {"h33_7": 3e-3}
+# cfg3 with gen_bias_init = -1.5: decoder linear_0/w sits at 6.2e-3 against the rounding-model oracle (every other tensor < 2e-3).
+# The same tensor is at 4.9e-3 at the default knobs on the same weights and inputs, under every launch plan: mask flips of
+# single decoder units; the oracle in fp32 instead of fp64 under the rounding model moves it by only 1.7e-4 here, so the flips
+# are not reproduced on the CPU.  Bounded for this case alone.
+MODEL_TENSOR_BOUND[("cfg3", "gen_bias_init=-1.5")] = 8e-3
+# bf16 against the EXACT oracle at one row of the cfg4 model: the oracle under the rounding model itself is 0.1151 away from the
+# exact one (encoder_gmm linear_1/w); the CUDA path measures 0.1151 and equals the rounding-model oracle to 0.0 (B200).
+GRAD_BF16_EXACT_BY_B = {1: 0.15}
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out")
 
 
@@ -51,19 +62,21 @@ def _record(name, obj):
         pass
 
 
-def _check_bf16(name, objective="reference", tag=""):
-    terr, gerr, ref = run_parity(CONFIGS[name], "bf16", objective=objective, want_ref=True)
-    bad = bf16_term_ok(terr, ref, TOL["bf16"])
+def _check_bf16(name, objective="reference", tag="", cfg=None):
+    """The bf16 bars of the module docstring on one case; `cfg` (default CONFIGS[name]) may carry hyperparameters."""
+    cfg = cfg or CONFIGS[name]
+    terr, gerr, ref = run_parity(cfg, "bf16", objective=objective, want_ref=True)
+    bad = bf16_term_ok(terr, ref, TERMS_BF16_TOL.get(name, TOL["bf16"]))
     assert not bad, (name, tag, "loss terms vs exact oracle (value, limit)", bad)
     assert max(gerr.values()) < GRAD_BF16_EXACT, (name, tag, gerr)
-    _, gerr_model = run_parity(CONFIGS[name], "bf16", rounding_model=Bf16Model(True), objective=objective)
+    _, gerr_model = run_parity(cfg, "bf16", rounding_model=Bf16Model(True), objective=objective)
     flat = sum(v * v for v in gerr_model.values()) ** 0.5 / len(gerr_model) ** 0.5
     _record(name, {"precision": "bf16", "objective": objective, "plan": tag, "terms_rel": terr, "terms_ref": ref,
                    "grad_vs_exact_max": max(gerr.values()), "grad_vs_model_max": max(gerr_model.values()), "grad_vs_model_rms": flat,
                    "grad_vs_model": gerr_model, "grad_vs_exact": gerr})
     assert flat < 1.5 * TOL["bf16"], (name, tag, "rms over tensors vs bf16 rounding model", flat)
     for k, v in gerr_model.items():
-        assert v < MODEL_TENSOR_BOUND.get(name, 3 * TOL["bf16"]), (name, tag, "vs bf16 rounding model", k, v)
+        assert v < MODEL_TENSOR_BOUND.get((name, tag), MODEL_TENSOR_BOUND.get(name, 3 * TOL["bf16"])), (name, tag, "vs bf16 rounding model", k, v)
 
 
 @pytest.mark.parametrize("name", list(CONFIGS))
@@ -93,14 +106,19 @@ def test_parity_bf16(name):
 # chained-GEMM launches with the heads as kernels in between; 8192 = heads as row jobs, the whole pass in ONE launch
 # (the default from 4096 samples up); 512 = no chaining, one launch per GEMM; 8192|4096 = one launch, weight gradients
 # not spread into the dependency bubbles.
+# the dispatch-boundary shapes of helpers.CONFIGS (heads, padded strides) run under every plan as well
+EDGE_SHAPES = ["k1_gmvae", "k16_gmvae", "k32_gmvae", "k33_gmvae", "k128_gmvae", "k128_gmp", "z1_vae", "z3_gmvae", "z65_gmp",
+               "z256_gmvae", "z260_gmvae", "z260_vae", "h33_7", "h129_gmp", "d97", "m_h36_20_k33", "m_k128_z8"]
+
+
 @pytest.mark.parametrize("flags", ["8192", "512", "12288"])
-@pytest.mark.parametrize("name", ["cfg1", "cfg3", "tiny_gmvae", "nohidden_gmvae", "run_train_sh", "cfg5_small", "k20_ragged"])
+@pytest.mark.parametrize("name", ["cfg1", "cfg3", "tiny_gmvae", "nohidden_gmvae", "run_train_sh", "cfg5_small", "k20_ragged"] + EDGE_SHAPES)
 def test_parity_bf16_launch_plans(name, flags, monkeypatch):
     monkeypatch.setenv("GMVAE_DEBUG_FLAGS", flags)
     _check_bf16(name, tag="flags=" + flags)
 
 
-MARGINAL_CASES = ["tiny_gmvae", "cfg3", "run_train_sh", "cfg5_small", "k20_ragged"]
+MARGINAL_CASES = ["tiny_gmvae", "cfg3", "run_train_sh", "cfg5_small", "k20_ragged", "m_h36_20_k33", "m_k128_z8"]
 
 
 @pytest.mark.parametrize("chunk_rows", [0, 96])
@@ -424,6 +442,34 @@ def test_full_size_parity_vs_oracle():
     assert flat < 1.5 * TOL["bf16"], ("rms over tensors vs bf16 rounding model", flat)
     for k, v in gerr_model.items():
         assert v < 3 * TOL["bf16"], ("vs bf16 rounding model", k, v)
+
+
+# Batch sizes around the plan switch of the cfg4 model: one row, one row short of 4 096 (the last batch on five chained launches),
+# 4 096 (row jobs and CTA pairs from here on), 4 097 (a one-row tail block)
+def _check_at(cfg, B, name, tag=""):
+    """bf16 bars of the small cases on one forward_backward of `cfg`'s model (cfg4's widths) over B rows of the full-size inputs:
+    terms against the exact oracle, tensors against the exact and the rounding-model one.  Only the bf16 path changes plan with
+    the batch (row jobs and CTA pairs from 4 096 rows); test_multi_row_block_fp32_mode covers the fp32 mode on many rows.  (The
+    fp32 mode is not held to 1e-5 here: on 4 097 or 5 000 of these rows the oracle evaluated in fp32 itself differs from the fp64
+    one by 3.7e-5 to 3.6e-4 on single tensors, ReLU masks that fp32 arithmetic decides differently.)"""
+    terr, gerr, ref = _parity_at(cfg, "bf16", B)
+    _, gerr_model, _ = _parity_at(cfg, "bf16", B, rounding_model=Bf16Model(True))
+    flat = sum(v * v for v in gerr_model.values()) ** 0.5 / len(gerr_model) ** 0.5
+    _record(name, {"precision": "bf16", "plan": tag, "terms_rel": terr, "terms_ref": ref, "grad_vs_exact_max": max(gerr.values()),
+                   "grad_vs_model_max": max(gerr_model.values()), "grad_vs_model_rms": flat, "grad_vs_model": gerr_model})
+    bad = bf16_term_ok(terr, ref, TOL["bf16"])
+    assert not bad, (name, tag, bad)
+    assert max(gerr.values()) < GRAD_BF16_EXACT_BY_B.get(B, GRAD_BF16_EXACT), (name, tag, gerr)
+    assert flat < 1.5 * TOL["bf16"], (name, tag, flat)
+    for k, v in gerr_model.items():
+        assert v < 3 * TOL["bf16"], (name, tag, k, v)
+
+
+@pytest.mark.parametrize("flags", ["0", "8192", "512"])
+@pytest.mark.parametrize("B", [1, 4095, 4096, 4097])
+def test_cfg4_model_batch_edges(B, flags, monkeypatch):
+    monkeypatch.setenv("GMVAE_DEBUG_FLAGS", flags)
+    _check_at(FULL, B, f"cfg4_B{B}", "flags=" + flags)
 
 
 @pytest.mark.parametrize("flags", ["0", "12288", "512"])
