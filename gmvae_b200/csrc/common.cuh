@@ -95,6 +95,12 @@ __device__ __forceinline__ float sigmoid_f(float t) {
   return t >= 0.f ? s : e * s;
 }
 
+// lo = log(sum_k exp(l_k - m)), m = max_k l_k, from `rest` = the sum of exp(l_k - m) over the entries below the max and `nmax` =
+// the number of entries equal to it: log1p(rest + nmax - 1).  The log-probabilities are then (l_k - m) - lo, never l_k - (m + lo).
+// When the softmax is nearly one-hot (rest ~ 1e-7) both other forms lose lo: 1 + rest rounds it away, and so does m + lo at ulp(m),
+// and q(y|x)'s entropy with it (relative 1e-3 at margins of 16 nats and logits of 20).
+__device__ __forceinline__ float lse_above_max(float rest, float nmax) { return log1pf(rest + (nmax - 1.f)); }
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -130,14 +136,19 @@ __device__ __forceinline__ float block_sum(float v, float* scratch) {
 enum { ACC_NLL = 0, ACC_KL = 32, ACC_NENT = 64, ACC_PER_TERM = 32, ACC_SLOTS = 96 };
 // Deterministic mode (gmvae_config::deterministic): sums whose addends arrive in no fixed order are taken in fixed point, as
 // int64 multiples of 2^-FX_SHIFT.  Integer addition is associative, so the total does not depend on the order of arrival; the
-// reduction step (det_reduce_kernel) converts it to fp32.  Resolution 1.5e-11 per addend.  Sum i lives in fx[2i]; fx[2i + 1]
-// flags an addend that is not finite or beyond +-2^26 (whose fixed-point form would saturate), and the reduction step then
-// writes NaN, as a NaN addend would have made of the default mode's float sum.  A sum of in-range addends beyond +-2^27 wraps
-// unflagged; the sums taken this way (loss terms, VAE_GMP prior gradients: means over the batch) stay far below that.
-enum { FX_SHIFT = 36 };
+// reduction step (det_reduce_kernel) converts it to fp32.  Resolution 1.5e-11 per addend, range +-2^27.  Sum i takes FX_WORDS
+// words at fx[FX_WORDS * i]: that fine sum; a flag word (bit 0: an addend that is not finite or beyond +-2^62, and the
+// reduction step writes NaN, as a NaN addend would have made of the default mode's float sum; bit 1: an addend beyond +-2^26,
+// which the fine sum leaves out); and the coarse sum of the addends rounded to integers, range +-2^63.  The reduction step
+// takes the coarse sum when bit 1 is set or the coarse total is 2^26 or more (the fine sum may have wrapped; a loss term of
+// a model whose posterior scales are far tighter than its prior's reaches 1e9 nats), and the fine sum otherwise.
+enum { FX_SHIFT = 36, FX_WORDS = 3 };
 __device__ __forceinline__ void fx_add(unsigned long long* fx, int i, float v) {
-  if (fabsf(v) < 67108864.f) atomicAdd(fx + 2 * i, (unsigned long long)__float2ll_rn(v * (float)(1ull << FX_SHIFT)));   // two's complement
-  else atomicOr(fx + 2 * i + 1, 1ull);                                                                                 // also NaN
+  unsigned long long* s = fx + FX_WORDS * i;
+  if (!(fabsf(v) < 4.611686e18f)) { atomicOr(s + 1, 1ull); return; }                                    // also NaN
+  if (fabsf(v) < 67108864.f) atomicAdd(s, (unsigned long long)__float2ll_rn(v * (float)(1ull << FX_SHIFT)));   // two's complement
+  else atomicOr(s + 1, 2ull);
+  atomicAdd(s + 2, (unsigned long long)__float2ll_rn(v));
 }
 // The training step passes the accumulator base with bit 0 set in deterministic mode: it then points at the fixed-point sums
 // above, one per term (index term / ACC_PER_TERM).

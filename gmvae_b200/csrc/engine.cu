@@ -398,7 +398,7 @@ static int plan(gmvae_handle* h) {
       for (const Linear& l : m->layers) cols += l.out;
     h->det_part_cap = cols * DET_ROW_BLOCKS;
     plan_buf(h, "det.part", (size_t)h->det_part_cap * 4);
-    plan_buf(h, "det.fx", (size_t)(3 + (c.model == GMVAE_MODEL_VAE_GMP ? K + 2 * K * Z : 0)) * 16);
+    plan_buf(h, "det.fx", (size_t)(3 + (c.model == GMVAE_MODEL_VAE_GMP ? K + 2 * K * Z : 0)) * 8 * FX_WORDS);
     // k-split slices of every weight gradient, for max_batch (the split count grows with the batch) in either plan
     h->det_wg_cap = 0;
     for (const Mlp* m : {&h->decoder, &h->encoder, &h->encoder_y, &h->prior_gmm})
@@ -1266,14 +1266,14 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
   unsigned long long* fx = h->det ? h->buf<unsigned long long>("det.fx") : nullptr;
   if (h->det) {
     const int nfx = 3 + (c.model == GMVAE_MODEL_VAE_GMP ? K + 2 * K * Z : 0);
-    GM_CHECK_CUDA(cudaMemsetAsync(fx, 0, (size_t)nfx * 16, st));
+    GM_CHECK_CUDA(cudaMemsetAsync(fx, 0, (size_t)nfx * 8 * FX_WORDS, st));
     acc = acc_fixed_tag(fx);
     h->det_segs.clear(); h->det_colsums.clear(); h->det_part_next = 0; h->det_wg_next = 0;
     h->det_segs.push_back(DetSeg{h->grads + h->n_params, nullptr, fx, 0, 3, 1, 0, ACC_PER_TERM, 0, 0});   // slot 0 of each term
     if (c.model == GMVAE_MODEL_VAE_GMP) {   // fx sums 3 ..: [K mixture logits | K*Z loc | K*Z raw_scale_diag] (gmp_prior_kernel)
-      h->det_segs.push_back(DetSeg{h->grads + h->mix_off, nullptr, fx + 2 * 3, 0, 1, K, 0, 0, 0, 0});
-      h->det_segs.push_back(DetSeg{h->grads + h->loc_off, nullptr, fx + 2 * (3 + K), 0, 1, K * Z, 0, 0, 0, 0});
-      h->det_segs.push_back(DetSeg{h->grads + h->raw_scale_off, nullptr, fx + 2 * (3 + K + K * Z), 0, 1, K * Z, 0, 0, 0, 0});
+      h->det_segs.push_back(DetSeg{h->grads + h->mix_off, nullptr, fx + FX_WORDS * 3, 0, 1, K, 0, 0, 0, 0});
+      h->det_segs.push_back(DetSeg{h->grads + h->loc_off, nullptr, fx + FX_WORDS * (3 + K), 0, 1, K * Z, 0, 0, 0, 0});
+      h->det_segs.push_back(DetSeg{h->grads + h->raw_scale_off, nullptr, fx + FX_WORDS * (3 + K + K * Z), 0, 1, K * Z, 0, 0, 0, 0});
     }
   }
 
@@ -1327,7 +1327,7 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
     GM_CHECK_CUDA(launch_k(gmp_prior_kernel, dim3((B + warps - 1) / warps), dim3(warps * 32), warps * K * sizeof(float), st, true,
                            (const float*)z_f32, (const float*)(h->params + h->loc_off), (const float*)(h->params + h->raw_scale_off),
                            (const float*)(h->params + h->mix_off), B, K, Z, inv_bg, dz_prior, h->grads + h->loc_off,
-                           h->grads + h->raw_scale_off, h->grads + h->mix_off, acc, fx ? fx + 2 * 3 : nullptr));
+                           h->grads + h->raw_scale_off, h->grads + h->mix_off, acc, fx ? fx + FX_WORDS * 3 : nullptr));
     GM_LAUNCHED(h, st, PC_HEADS);
   }
   // decoder: hidden layers, then logits fused with the Bernoulli log-likelihood (and db of that layer)

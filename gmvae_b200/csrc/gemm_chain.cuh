@@ -186,13 +186,21 @@ __device__ __forceinline__ void pack16(const float* v, uint4& lo, uint4& hi) {
 // Warp-collective (all 32 lanes call; `valid` masks rows beyond the batch) and deliberately NOT inlined: the thin
 // GEMM jobs that host them sit on the critical path of the chain and must not inherit their register footprint.
 // forward: lg = logits (with bias).  Writes y (fp32 + zero-padded bf16 operand row), returns sum_k p log p of the row.
-// Math of the heads inside the chained kernel (bf16 training step only): fast intrinsics.  exp / log arguments are logits
-// and softmax sums of magnitude O(1-100): __expf / __logf are good to ~2 ulp there (abs error of log(1+e), 1+e in (1,2]:
-// ~1e-7), far inside the bf16 storage the results go to.  The fp32 validation mode never runs these (kernels.cuh heads).
+// Math of the heads inside the chained kernel (bf16 training step only): fast intrinsics.  The fp32 validation mode never
+// runs these (kernels.cuh heads).  __expf is good to ~2 ulp relative.  __logf(s) is good to an ABSOLUTE ~1e-7 near s = 1,
+// which is enough where the result is O(1) or is added to one: the BCE loss, and the y head's lse = ml + log(sl), whose
+// absolute error of ~ulp(ml) per row stays far below the bf16 bars even when q(y|x) is nearly one-hot.  It is not
+// enough for softplus(t) = log(1 + e), e = exp(t), on its own as a scale: below t ~ -5 the sum 1 + e drops the low bits of
+// e (relative error 5e-4 at sigma = 1e-4, 6e-2 at 1e-6, and sigma = 0 -- log 0, 1/0 -- below 6e-8), so the z heads take
+// log1p_fast, which is accurate to ~1 ulp relative for small e as well.
 __device__ __forceinline__ float exp2f_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float lg2_approx(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float fast_softplus(float t) { return fmaxf(t, 0.f) + __logf(1.f + __expf(-fabsf(t))); }
+// log(1 + e) for e in [0, 1]: below 2^-7 the series e (1 - e/2 + e^2/3) (truncation e^4/4 < 2^-23 e), above it __logf(1 + e)
+__device__ __forceinline__ float log1p_fast(float e) {
+  return e < 0.0078125f ? e * fmaf(e, fmaf(e, 0.33333334f, -0.5f), 1.f) : __logf(1.f + e);
+}
+__device__ __forceinline__ float fast_softplus(float t) { return fmaxf(t, 0.f) + log1p_fast(__expf(-fabsf(t))); }
 __device__ __forceinline__ float fast_sigmoid(float t) {
   const float e = __expf(-fabsf(t));
   const float s = __fdividef(1.f, 1.f + e);
@@ -786,7 +794,7 @@ __device__ __forceinline__ void chain_rows_job(const ChainJob& J, int* counters,
           // softplus(t) and sigmoid(t) from ONE exponential: e = exp(-|t|), softplus = max(t,0) + log(1+e), sigmoid = (t>=0 ? 1 : e)/(1+e)
           const float tq = RAW[q] + prm.c;
           const float eq = __expf(-fabsf(tq)), iq = __fdividef(1.f, 1.f + eq);
-          const float spq = fmaxf(tq, 0.f) + __logf(1.f + eq);
+          const float spq = fmaxf(tq, 0.f) + log1p_fast(eq);
           const float sgm_q = tq >= 0.f ? iq : eq * iq;
           const float sg = fmaxf(spq, prm.sigma_min);
           const float z = fmaf(sg, E[q], MU[q]);
@@ -797,7 +805,7 @@ __device__ __forceinline__ void chain_rows_job(const ChainJob& J, int* counters,
           } else {
             const float tp = RP[q] + prm.c;
             const float ep = __expf(-fabsf(tp)), ip = __fdividef(1.f, 1.f + ep);
-            const float spp = fmaxf(tp, 0.f) + __logf(1.f + ep);
+            const float spp = fmaxf(tp, 0.f) + log1p_fast(ep);
             const float sgm_p = tp >= 0.f ? ip : ep * ip;
             const float sp = fmaxf(spp, prm.sigma_min);
             const float d = z - MP[q];

@@ -146,19 +146,19 @@ __global__ void head_y_fwd_kernel(const float* __restrict__ logits, const float*
       ml = fmaxf(ml, l[i]); ma = fmaxf(ma, a[i]);
     }
     ml = warp_max(ml); ma = warp_max(ma);
-    float sl = 0.f, sa = 0.f;
+    float sl = 0.f, nm = 0.f, sa = 0.f;
 #pragma unroll
     for (int i = 0; i < HEAD_MAXK / 32; ++i) {
       int k = lane + 32 * i;
-      if (k < K) { sl += expf(l[i] - ml); sa += expf(a[i] - ma); }
+      if (k < K) { if (l[i] == ml) nm += 1.f; else sl += expf(l[i] - ml); sa += expf(a[i] - ma); }
     }
-    sl = warp_sum(sl); sa = warp_sum(sa);
-    const float lse = ml + logf(sl), inv_sa = 1.f / sa;
+    sl = warp_sum(sl); nm = warp_sum(nm); sa = warp_sum(sa);
+    const float lo = lse_above_max(sl, nm), inv_sa = 1.f / sa;
 #pragma unroll
     for (int i = 0; i < HEAD_MAXK / 32; ++i) {
       int k = lane + 32 * i;
       if (k < K) {
-        float logp = l[i] - lse;
+        float logp = (l[i] - ml) - lo;
         ent += expf(logp) * logp;
         float y = expf(a[i] - ma) * inv_sa;
         y_f32[(int64_t)row * K + k] = y;
@@ -201,22 +201,22 @@ __global__ void head_y_bwd_kernel(const float* __restrict__ logits, const float*
     ydy += y[i] * g[i];
   }
   ml = warp_max(ml); ydy = warp_sum(ydy);
-  float sl = 0.f;
+  float sl = 0.f, nm = 0.f;
 #pragma unroll
   for (int i = 0; i < HEAD_MAXK / 32; ++i)
-    if (lane + 32 * i < K) sl += expf(l[i] - ml);
-  sl = warp_sum(sl);
-  const float lse = ml + logf(sl);
+    if (lane + 32 * i < K) { if (l[i] == ml) nm += 1.f; else sl += expf(l[i] - ml); }
+  sl = warp_sum(sl); nm = warp_sum(nm);
+  const float lo = lse_above_max(sl, nm);
   float plogp = 0.f;
 #pragma unroll
   for (int i = 0; i < HEAD_MAXK / 32; ++i)
-    if (lane + 32 * i < K) { float lp = l[i] - lse; plogp += expf(lp) * lp; }
+    if (lane + 32 * i < K) { float lp = (l[i] - ml) - lo; plogp += expf(lp) * lp; }
   plogp = warp_sum(plogp);
 #pragma unroll
   for (int i = 0; i < HEAD_MAXK / 32; ++i) {
     int k = lane + 32 * i;
     if (k < K) {
-      float lp = l[i] - lse;
+      float lp = (l[i] - ml) - lo;
       ActT o = from_f32<ActT>(y[i] * (g[i] - ydy) * inv_T + expf(lp) * (lp - plogp) * inv_bg);
       dlogits[(int64_t)row * ld_out + k] = o;
       cs[i] += to_f32<ActT>(o);
@@ -532,17 +532,17 @@ __global__ void head_y_fwd_row_kernel(const float* __restrict__ logits, const fl
       }
       ml = fmaxf(ml, l[k]); ma = fmaxf(ma, a[k]);
     }
-    float sl = 0.f, sa = 0.f;
+    float sl = 0.f, nm = 0.f, sa = 0.f;
 #pragma unroll
     for (int k = 0; k < 16; ++k)
-      if (k < K) { a[k] = expf(a[k] - ma); sl += expf(l[k] - ml); sa += a[k]; }
-    const float lse = ml + logf(sl), inv_sa = 1.f / sa;
+      if (k < K) { a[k] = expf(a[k] - ma); if (l[k] == ml) nm += 1.f; else sl += expf(l[k] - ml); sa += a[k]; }
+    const float lo = lse_above_max(sl, nm), inv_sa = 1.f / sa;
     float y[16];
 #pragma unroll
     for (int k = 0; k < 16; ++k) {
       y[k] = 0.f;
       if (k < K) {
-        const float logp = l[k] - lse;
+        const float logp = (l[k] - ml) - lo;
         ent += expf(logp) * logp;
         y[k] = a[k] * inv_sa;
         y_f32[(int64_t)row * K + k] = y[k];
@@ -583,15 +583,15 @@ __global__ void head_y_bwd_row_kernel(const float* __restrict__ logits, const fl
       ml = fmaxf(ml, l[k]);
       ydy += y[k] * g[k];
     }
-    float sl = 0.f;
+    float sl = 0.f, nm = 0.f;
 #pragma unroll
     for (int k = 0; k < 16; ++k)
-      if (k < K) sl += expf(l[k] - ml);
-    const float lse = ml + logf(sl);
+      if (k < K) { if (l[k] == ml) nm += 1.f; else sl += expf(l[k] - ml); }
+    const float lo = lse_above_max(sl, nm);
     float plogp = 0.f;
 #pragma unroll
     for (int k = 0; k < 16; ++k)
-      if (k < K) { l[k] -= lse; plogp += expf(l[k]) * l[k]; }
+      if (k < K) { l[k] = (l[k] - ml) - lo; plogp += expf(l[k]) * l[k]; }
     float o[16];
 #pragma unroll
     for (int k = 0; k < 16; ++k) {
@@ -999,22 +999,22 @@ __global__ void head_y_m_bwd_kernel(const float* __restrict__ logits, const floa
     for (int i = 0; i < HEAD_MAXK / 32; ++i) cc[i] = (float)(cd[i] - pcd);
     const float pc = 0.f;
     ml = warp_max(ml);
-    float sl = 0.f;
+    float sl = 0.f, nm = 0.f;
 #pragma unroll
     for (int i = 0; i < HEAD_MAXK / 32; ++i)
-      if (lane + 32 * i < K) sl += expf(l[i] - ml);
-    sl = warp_sum(sl);
-    const float lse = ml + logf(sl);
+      if (lane + 32 * i < K) { if (l[i] == ml) nm += 1.f; else sl += expf(l[i] - ml); }
+    sl = warp_sum(sl); nm = warp_sum(nm);
+    const float lo = lse_above_max(sl, nm);
     float plogp = 0.f;
 #pragma unroll
     for (int i = 0; i < HEAD_MAXK / 32; ++i)
-      if (lane + 32 * i < K) { float lp = l[i] - lse; plogp += expf(lp) * lp; }
+      if (lane + 32 * i < K) { float lp = (l[i] - ml) - lo; plogp += expf(lp) * lp; }
     plogp = warp_sum(plogp);
 #pragma unroll
     for (int i = 0; i < HEAD_MAXK / 32; ++i) {
       int k = lane + 32 * i;
       if (k < K) {
-        float lp = l[i] - lse;
+        float lp = (l[i] - ml) - lo;
         ActT o = from_f32<ActT>((p[i] * (cc[i] - pc) + expf(lp) * (lp - plogp)) * inv_bg);
         dlogits[(int64_t)row * ld_out + k] = o;
         cs[i] += to_f32<ActT>(o);
@@ -1090,7 +1090,11 @@ __global__ void det_reduce_kernel(const __grid_constant__ DetSegs segs) {
     const int r = (int)(i / g.cols), c = (int)(i % g.cols);
     float v = 0.f;
     if (g.fx) {
-      v = g.fx[2 * i + 1] ? __int_as_float(0x7fffffff) : (float)((double)(long long)g.fx[2 * i] * (1.0 / (double)(1ull << FX_SHIFT)));
+      const unsigned long long* f = g.fx + FX_WORDS * i;
+      const long long coarse = (long long)f[2];
+      v = (f[1] & 1ull) ? __int_as_float(0x7fffffff)
+        : ((f[1] & 2ull) || coarse >= (1ll << 26) || coarse <= -(1ll << 26)) ? (float)coarse
+        : (float)((double)(long long)f[0] * (1.0 / (double)(1ull << FX_SHIFT)));
     } else {
       const float* p = g.part + (long long)r * g.ld_part + c;
       for (int s = 0; s < g.nparts; ++s) v += p[(long long)s * g.part_stride];
