@@ -374,6 +374,9 @@ static int plan(gmvae_handle* h) {
       plan_buf(h, "dxproj", Bfull * round_up((int)H0, 8) * asz);
       plan_buf(h, "rec", Bfull * K * 8);
       plan_buf(h, "klrow", Bfull * K * 4);
+      // the fp32 validation mode's y W[D:] + b of gmvae_encode / gmvae_condition(encoder_gmm): [max_batch, H0] fp32 like the
+      // x-projection, which only the training step uses
+      h->bufs["pre_y"] = h->bufs["xproj"];
     } else {
       plan_buf(h, "prior_out", Bfull * 2 * Z * 4);
       plan_buf(h, "d_prior_out", Bfull * round_up(2 * Z, 8) * asz);
@@ -1157,7 +1160,8 @@ static int forward_encoder(gmvae_handle* h, const uint8_t* x_u8, int B, float in
     }
     // p(z|y): one linear K -> 2Z (gmvae.py:243, 321-327).  Issued after encoder_gmm's first layer: in the chained kernel that
     // layer starts on its x segment while the y head is still finishing, and y is complete by the time this thin job runs.
-    {
+    // Objective M reaches here only through gmvae_encode, which does not read p(z|y); its handles plan no prior_out.
+    if (c.objective == GMVAE_OBJECTIVE_REFERENCE) {
       const Linear& l = h->prior_gmm.layers[0];
       EpiStore<float> epi{prior_out, (int64_t)2 * Z, h->params + l.b_off, nullptr, 0, 0, 1.f};
       GM_TRY(lin_fwd<A>(h, y_act, Kp, B, view(h, l), epi, st));
@@ -2188,13 +2192,13 @@ static int condition_impl(gmvae_handle* h, int which, const float* in1, const fl
   }
   if (which == GMVAE_COND_PRIOR_GMM) {                        // p(z|y): one linear K -> 2Z
     GM_REQUIRE(gm, "prior_gmm exists in the GMVAE only");
-    A* y_act = h->buf<A>("y_act"); float* prior_out = h->buf<float>("prior_out");
-    GM_REQUIRE(prior_out != nullptr, "gmvae_condition(prior_gmm) needs a handle created with objective=reference");
+    // [mu|raw] into enc_out, which every handle plans (objective-M handles have no prior_out)
+    A* y_act = h->buf<A>("y_act"); float* outs = h->buf<float>("enc_out");
     GM_TRY(to_act(in1, K, y_act, Kp));
     const Linear& l = h->prior_gmm.layers[0];
-    EpiStore<float> epi{prior_out, (int64_t)2 * Z, h->params + l.b_off, nullptr, 0, 0, 1.f};
+    EpiStore<float> epi{outs, (int64_t)2 * Z, h->params + l.b_off, nullptr, 0, 0, 1.f};
     GM_TRY(lin_fwd<A>(h, y_act, Kp, n, view(h, l), epi, st));
-    return normal_out(prior_out);
+    return normal_out(outs);
   }
   GM_REQUIRE(which == GMVAE_COND_ENCODER, "unknown conditional distribution");
   MlpBufs<A> enc = mlp_bufs<A>(h, h->encoder);
@@ -2207,7 +2211,6 @@ static int condition_impl(gmvae_handle* h, int which, const float* in1, const fl
   }
   // q(z|x,y): [x,y] W = x W[:D] + y W[D:]  (no concat, base.py:66)
   GM_REQUIRE(in2 != nullptr, "encoder_gmm takes (x, y)");
-  GM_REQUIRE(c.objective == GMVAE_OBJECTIVE_REFERENCE, "gmvae_condition(encoder_gmm) needs a handle created with objective=reference");
   A* y_act = h->buf<A>("y_act");
   GM_TRY(to_act(in2, K, y_act, Kp));
   const Linear& enc_l0 = h->encoder.layers[0];
@@ -2241,6 +2244,26 @@ static int condition_impl(gmvae_handle* h, int which, const float* in1, const fl
   return normal_out(enc_out);
 }
 
+// Rows one pass of an inference entry point may hold.  An objective-M handle plans its per-component buffers (z_act, enc_out,
+// the decoder's and encoder_gmm's hidden layers) for chunk_samples * K rows, which can be fewer than max_batch; every other
+// buffer holds max_batch rows or more.
+static int infer_rows(const gmvae_handle* h) {
+  if (h->cfg.objective != GMVAE_OBJECTIVE_MARGINAL) return h->cfg.max_batch;
+  return (int)std::min<int64_t>((int64_t)h->chunk_samples * h->K, INT32_MAX);
+}
+
+// Runs pass(r0, rows) over rows [0, n) in slices of at most infer_rows(h) rows, in order on the caller's stream.  A row's
+// result depends on that row alone, so the slices give what one pass over n rows would.
+template <class F>
+static int for_row_slices(const gmvae_handle* h, int n, F pass) {
+  const int cap = infer_rows(h);
+  for (int r0 = 0; r0 < n; r0 += cap) GM_TRY(pass(r0, std::min(cap, n - r0)));
+  return 0;
+}
+
+// rows [r0, ...) of a row-major matrix `cols` wide, or null
+template <typename T> static T* rows_from(T* p, int r0, int cols) { return p ? p + (int64_t)r0 * cols : nullptr; }
+
 extern "C" {
 
 int gmvae_encode(gmvae_handle* h, const uint8_t* x_u8, int batch, const float* eps, const float* gumbel_u, float* logits_y, float* z_mean,
@@ -2249,9 +2272,14 @@ int gmvae_encode(gmvae_handle* h, const uint8_t* x_u8, int batch, const float* e
   GM_TRY(check_ready(h));
   GM_REQUIRE(x_u8 && z_mean && z_sample, "null argument");
   GM_REQUIRE(batch > 0 && batch <= h->cfg.max_batch, "batch must be in [1, max_batch]");
-  GM_REQUIRE(h->cfg.objective == GMVAE_OBJECTIVE_REFERENCE, "gmvae_encode needs a handle created with objective=reference");
-  if (h->bf16_mode()) return encode_impl<bf16>(h, x_u8, batch, eps, gumbel_u, logits_y, z_mean, z_sample, (cudaStream_t)stream);
-  return encode_impl<float>(h, x_u8, batch, eps, gumbel_u, logits_y, z_mean, z_sample, (cudaStream_t)stream);
+  const int D = h->D, Z = h->Z, K = h->K;
+  return for_row_slices(h, batch, [&](int r0, int n) {
+    const uint8_t* x = rows_from(x_u8, r0, D);
+    const float* e = rows_from(eps, r0, Z); const float* u = rows_from(gumbel_u, r0, K);
+    float* ly = rows_from(logits_y, r0, K); float* zm = rows_from(z_mean, r0, Z); float* zs = rows_from(z_sample, r0, Z);
+    if (h->bf16_mode()) return encode_impl<bf16>(h, x, n, e, u, ly, zm, zs, (cudaStream_t)stream);
+    return encode_impl<float>(h, x, n, e, u, ly, zm, zs, (cudaStream_t)stream);
+  });
 }
 int gmvae_condition(gmvae_handle* h, int which, const float* in1, const float* in2, int n, float* out_a, float* out_b, void* stream) {
   DeviceGuard dev_guard(h);
@@ -2260,8 +2288,15 @@ int gmvae_condition(gmvae_handle* h, int which, const float* in1, const float* i
   GM_REQUIRE(n > 0 && n <= h->cfg.max_batch, "n must be in [1, max_batch]");
   GM_REQUIRE(which >= 0 && which <= 3, "unknown conditional distribution");
   GM_REQUIRE(out_b || which == GMVAE_COND_DECODER || which == GMVAE_COND_ENCODER_Y, "a ConditionalNormal returns (mu, sigma): out_b is null");
-  if (h->bf16_mode()) return condition_impl<bf16>(h, which, in1, in2, n, out_a, out_b, (cudaStream_t)stream);
-  return condition_impl<float>(h, which, in1, in2, n, out_a, out_b, (cudaStream_t)stream);
+  // row widths of in1 and out_a (in2 = y and out_b = sigma are K and Z wide wherever they are used)
+  const int w_in1[4] = {h->Z, h->D, h->D, h->K};
+  const int w_out[4] = {h->D, h->Z, h->K, h->Z};
+  return for_row_slices(h, n, [&](int r0, int rows) {
+    const float* a1 = rows_from(in1, r0, w_in1[which]); const float* a2 = rows_from(in2, r0, h->K);
+    float* oa = rows_from(out_a, r0, w_out[which]); float* ob = rows_from(out_b, r0, h->Z);
+    if (h->bf16_mode()) return condition_impl<bf16>(h, which, a1, a2, rows, oa, ob, (cudaStream_t)stream);
+    return condition_impl<float>(h, which, a1, a2, rows, oa, ob, (cudaStream_t)stream);
+  });
 }
 // sample / log_prob / mean of the distribution objects the Conditional* classes return (TFP semantics, SURVEY Appendix B.3-B.5)
 int gmvae_dist_normal_sample(const float* mu, const float* sigma, const float* eps, int64_t n, float* out, void* stream) {
@@ -2295,10 +2330,13 @@ int gmvae_decode(gmvae_handle* h, const float* z, int n, float* x_mean, void* st
   DeviceGuard dev_guard(h);
   GM_TRY(check_ready(h));
   GM_REQUIRE(z && x_mean, "null argument");
-  const int cap = h->cfg.objective == GMVAE_OBJECTIVE_MARGINAL ? h->chunk_samples * h->K : h->cfg.max_batch;
-  GM_REQUIRE(n > 0 && n <= cap, "n must be in [1, max_batch]");
-  if (h->bf16_mode()) return decode_impl<bf16>(h, z, n, x_mean, (cudaStream_t)stream);
-  return decode_impl<float>(h, z, n, x_mean, (cudaStream_t)stream);
+  // decode touches the per-component buffers only: an objective-M handle also takes one pass of up to chunk_samples * K rows
+  GM_REQUIRE(n > 0 && n <= std::max(h->cfg.max_batch, infer_rows(h)), "n must be in [1, max_batch]");
+  return for_row_slices(h, n, [&](int r0, int rows) {
+    const float* zz = rows_from(z, r0, h->Z); float* xm = rows_from(x_mean, r0, h->D);
+    if (h->bf16_mode()) return decode_impl<bf16>(h, zz, rows, xm, (cudaStream_t)stream);
+    return decode_impl<float>(h, zz, rows, xm, (cudaStream_t)stream);
+  });
 }
 int gmvae_prior_table(gmvae_handle* h, float* mu, float* sigma, void* stream) {
   DeviceGuard dev_guard(h);

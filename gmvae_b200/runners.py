@@ -205,7 +205,10 @@ def process_over_dataset(model, eng, batches, config):
 
 
 def run_eval(config, max_wait: Optional[float] = None):
-    """runners.py:235-458: one pass over `config.split`, loss summary, latent / prior-sample plots, image grids."""
+    """runners.py:235-458: one pass over `config.split`, loss summary, latent / prior-sample plots, image grids.
+    The loss is that of `run_model` on the engine `config.objective` builds: with `--objective=marginal`, the objective-M loss
+    (the K-way marginalised ELBO, DESIGN.md section 1), not the reference's one-sample estimate.  Both objectives share one
+    variable layout, so either can evaluate a checkpoint the other trained."""
     torch.manual_seed(config.random_seed or 0)
     if config.random_seed:
         np.random.seed(config.random_seed)

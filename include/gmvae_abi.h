@@ -159,9 +159,12 @@ GMVAE_API int gmvae_step_graph_launch(gmvae_handle* h, void* stream);
 
 /* Forward-only helpers behind the model classes' inference methods
  * (gmvae.py:109-188, vae.py:80-123).  out buffers are device float arrays.
- *   encode : x -> (optional) logits_y [batch,K], z_mean [batch,Z], z_sample [batch,Z]
+ *   encode : x -> (optional) logits_y [batch,K], z_mean [batch,Z], z_sample [batch,Z]; noise as in the step under objective R
+ *            (eps [batch,Z], gumbel_u [batch,K], each drawn on the device when NULL), on a handle of either objective
  *   decode : z [n,Z] -> Bernoulli mean sigmoid(logits) [n, data_size]
- *   prior  : GMVAE prior_gmm(one_hot(k)) table -> mu [K,Z], sigma [K,Z] */
+ *   prior  : GMVAE prior_gmm(one_hot(k)) table -> mu [K,Z], sigma [K,Z]
+ * batch / n may be anything in [1, max_batch] on every handle (decode on an objective-M handle: also up to its chunk of
+ * component rows, chunk_samples * K); where the handle's buffers hold fewer rows, the rows are processed in slices. */
 GMVAE_API int gmvae_encode(gmvae_handle* h, const uint8_t* x_u8, int batch, const float* eps,
                  const float* gumbel_u, float* logits_y, float* z_mean, float* z_sample,
                  void* stream);
@@ -174,7 +177,9 @@ GMVAE_API int gmvae_prior_table(gmvae_handle* h, float* mu, float* sigma, void* 
  *   GMVAE_COND_ENCODER   in1 = x [n,D] (in2 = y [n,K] for the GMVAE's encoder_gmm) -> out_a = mu, out_b = sigma [n,Z]
  *   GMVAE_COND_ENCODER_Y in1 = x [n,D]                    -> out_a = logits of q(y|x) [n,K]
  *   GMVAE_COND_PRIOR_GMM in1 = y [n,K]                    -> out_a = mu, out_b = sigma [n,Z]
- * with sigma = max(softplus(raw + raw_sigma_bias), sigma_min) (base.py:69-70).  The model accessors decoder(z), encoder(x),
+ * with sigma = max(softplus(raw + raw_sigma_bias), sigma_min) (base.py:69-70); y is any dense [n,K] matrix.  All four run on a
+ * handle of either objective, for any n in [1, max_batch] (in slices where its buffers hold fewer rows, as for encode).
+ * The model accessors decoder(z), encoder(x),
  * encoder_y(x), encoder_gmm(x,y), prior_gmm(y) (gmvae.py:49-107, vae.py:41-78) are these.
  * gmvae_dist_*: sample / log_prob / mean of the distributions those classes return (base.py:75-83, 138-146, 201-209):
  * MultivariateNormalDiag(loc, scale_diag), Independent(Bernoulli(logits), 1), RelaxedOneHotCategorical(T, logits).  Noise is
