@@ -2477,7 +2477,8 @@ int gmvae_debug_gemm(gmvae_handle* h, int impl, int transA, int transB, int M, i
   // A stored [M,K] (transA=0 -> K-major) or [K,M] (transA=1 -> MN-major);
   // B stored [K,N] (transB=0 -> MN-major) or [N,K] (transB=1 -> K-major).
   const bool a_mn = transA != 0, b_mn = transB == 0;
-  GM_REQUIRE(a_mn == b_mn, "debug hook covers K-major x K-major and MN-major x MN-major");
+  GM_REQUIRE(a_mn == b_mn || (!a_mn && b_mn),
+             "debug hook covers K-major x K-major, K-major x MN-major (forward) and MN-major x MN-major");
   const int64_t a_rows = a_mn ? K : M, a_cols = a_mn ? M : K, b_rows = b_mn ? K : N, b_cols = b_mn ? N : K;
   const int64_t lda = round_up((int)a_cols, 8), ldb = round_up((int)b_cols, 8);
   bf16 *a16 = nullptr, *b16 = nullptr;
@@ -2489,7 +2490,7 @@ int gmvae_debug_gemm(gmvae_handle* h, int impl, int transA, int transB, int M, i
   if (impl >= 2) {
     // traced run of a forward-style layer: out = relu(A B^T + bias) in bf16; the first 4096 int64 of C
     // receive CTA 0's clock64 stamps (16 per tile: see gemm_tc.cuh)
-    GM_REQUIRE(!a_mn && (size_t)M * N * 4 >= 4096 * 8, "trace needs K-major operands and a large enough C");
+    GM_REQUIRE(!a_mn && !b_mn && (size_t)M * N * 4 >= 4096 * 8, "trace needs K-major operands and a large enough C");
     bf16* o16 = nullptr; float* bias = nullptr; long long* tr = nullptr;
     GM_CHECK_CUDA(cudaMalloc(&o16, (size_t)M * round_up(N, 8) * 2));
     GM_CHECK_CUDA(cudaMalloc(&bias, (size_t)N * 4));
@@ -2513,7 +2514,11 @@ int gmvae_debug_gemm(gmvae_handle* h, int impl, int transA, int transB, int M, i
     GM_CHECK_CUDA(e);
     return 0;
   }
-  if (!a_mn) {
+  if (!a_mn && b_mn) {
+    // the forward orientation of lin_fwd: B = W[K, N] as stored; its rows beyond K lie outside the tensor map (read as zero)
+    tc::Operand a{a16, lda, M, kpad(K, lda)}, b{b16, ldb, N, K};
+    r = tc_dispatch_kk<EpiAtomicAdd, true>(h, a, b, nullptr, nullptr, M, N, epi, st);
+  } else if (!a_mn) {
     tc::Operand a{a16, lda, M, kpad(K, lda)}, b{b16, ldb, N, kpad(K, ldb)};
     r = tc_dispatch_kk(h, a, b, nullptr, nullptr, M, N, epi, st);
   } else {

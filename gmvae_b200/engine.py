@@ -247,8 +247,14 @@ class Engine:
         zm = torch.empty(B, Z, dtype=torch.float32, device=self.device)
         zs = torch.empty(B, Z, dtype=torch.float32, device=self.device)
         self._keep = [xu, e, u]
-        _lib.check(self.lib.gmvae_encode(self._h, xu.data_ptr(), B, _ptr(e), _ptr(u), _ptr(logits), zm.data_ptr(), zs.data_ptr(),
-                                         self._stream()), "gmvae_encode")
+        # gmvae_encode takes at most max_batch rows: larger batches go in slices, as in decode (rows are independent)
+        for i in range(0, B, self.max_batch):
+            n = min(self.max_batch, B - i)
+            ei = None if e is None else e[i:i + n]
+            ui = None if u is None else u[i:i + n]
+            li = None if logits is None else logits[i:i + n]
+            _lib.check(self.lib.gmvae_encode(self._h, xu[i:i + n].data_ptr(), n, _ptr(ei), _ptr(ui), _ptr(li), zm[i:i + n].data_ptr(),
+                                             zs[i:i + n].data_ptr(), self._stream()), "gmvae_encode")
         return logits, zm, zs
 
     def decode(self, z) -> torch.Tensor:
@@ -418,7 +424,10 @@ class Engine:
         return e, u
 
     def debug_gemm(self, impl: int, A: torch.Tensor, B: torch.Tensor, transA=False, transB=False, split_k=1) -> torch.Tensor:
-        """C = op(A) op(B) through the step's own GEMM kernels (impl 0 SIMT fp32, 1 tcgen05 bf16)."""
+        """C = op(A) op(B) through the step's own GEMM kernels (impl 0 SIMT fp32, 1 tcgen05 bf16).  impl 1 takes
+        (transA, transB) = (False, True): both operands K-major, the data-gradient GEMMs; (False, False): A K-major and B
+        MN-major, the forward GEMM of a layer outside the chained kernel (what encode / decode / condition run); and
+        (True, False): both MN-major, the weight-gradient GEMMs."""
         A = A.to(self.device, torch.float32).contiguous(); B = B.to(self.device, torch.float32).contiguous()
         M, K = (A.shape[1], A.shape[0]) if transA else A.shape
         N = B.shape[0] if transB else B.shape[1]

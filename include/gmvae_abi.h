@@ -213,7 +213,10 @@ GMVAE_API int gmvae_unpack_bits(gmvae_handle* h, const uint8_t* packed, int batc
 
 /* Kernel-level test hook: C[M,N] = A[M,K] * B[K,N] through the same GEMM kernels the step
  * uses (impl 0 = fp32 SIMT, 1 = tcgen05 bf16).  A, B, C are device float arrays, row-major;
- * transA/transB say the stored matrix is the transpose ([K,M] / [N,K]).  Used by tests/. */
+ * transA/transB say the stored matrix is the transpose ([K,M] / [N,K]).  impl 1 takes three of the four
+ * combinations: transA=0 transB=1 (both K-major: the data-gradient GEMMs), transA=0 transB=0 (A K-major, B
+ * MN-major: the forward GEMMs of the layers, dispatched to the tile widths inference uses) and transA=1
+ * transB=0 (both MN-major: the weight-gradient GEMMs).  Used by tests/. */
 GMVAE_API int gmvae_debug_gemm(gmvae_handle* h, int impl, int transA, int transB, int M, int N, int K,
                      const float* A, const float* B, float* C, int split_k, void* stream);
 
