@@ -1042,6 +1042,26 @@ static int mlp_backward(gmvae_handle* h, const Mlp& m, const MlpBufs<A>& b, cons
 }
 
 // ============================================================================ the step
+// q(y|x) head for HEAD_MAXK < K <= HEAD_WIDE_MAXK: the row width in registers is the smallest of 256 / 512 / 1024 that holds K
+template <typename A>
+static int head_y_wide_fwd(int K, const float* logits, const float* gum, int B, float inv_T, float inv_bg, float* y_f32, A* y_act, int ld_yact,
+                           float* acc, cudaStream_t st) {
+  auto kern = K <= 256 ? head_y_wide_fwd_kernel<A, 256> : K <= 512 ? head_y_wide_fwd_kernel<A, 512> : head_y_wide_fwd_kernel<A, 1024>;
+  const int rows = HEAD_WIDE_THREADS / 32;
+  GM_CHECK_CUDA(launch_k(kern, dim3((B + rows - 1) / rows), dim3(HEAD_WIDE_THREADS), 0, st, true, logits, gum, B, K, inv_T, inv_bg, y_f32, y_act,
+                         ld_yact, acc));
+  return 0;
+}
+template <typename A>
+static int head_y_wide_bwd(int K, const float* logits, const float* y_f32, const float* dy, int B, float inv_T, float inv_bg, A* dlogits,
+                           int ld_out, float* db, cudaStream_t st) {
+  auto kern = K <= 256 ? head_y_wide_bwd_kernel<A, 256> : K <= 512 ? head_y_wide_bwd_kernel<A, 512> : head_y_wide_bwd_kernel<A, 1024>;
+  const int rows = HEAD_WIDE_THREADS / 32;
+  GM_CHECK_CUDA(launch_k(kern, dim3(std::max(1, std::min(4 * tc::num_sms(), (B + rows - 1) / rows))), dim3(HEAD_WIDE_THREADS), 0, st, true, logits,
+                         y_f32, dy, B, K, inv_T, inv_bg, dlogits, ld_out, db));
+  return 0;
+}
+
 // Input conversion, noise and the encoder side of the forward pass (q(y|x), the relaxed sample y,
 // p(z|y), q(z|x,y) / q(z|x)) up to the encoder's [mu|raw] output.  Shared by the training step and by
 // gmvae_encode (reconstruct_images / transform of the model classes).
@@ -1126,6 +1146,8 @@ static int forward_encoder(gmvae_handle* h, const uint8_t* x_u8, int B, float in
     if (std::is_same<A, bf16>::value && K <= 16 && Kp <= 16) {
       GM_CHECK_CUDA(launch_k(head_y_fwd_row_kernel, dim3((B + 127) / 128), dim3(128), 0, st, true, (const float*)logits_y, u, B, K,
                              1.f / c.temperature, inv_bg, y_f32, reinterpret_cast<bf16*>(y_act), Kp, acc));
+    } else if (K > HEAD_MAXK) {
+      GM_TRY(head_y_wide_fwd<A>(K, logits_y, u, B, 1.f / c.temperature, inv_bg, y_f32, y_act, Kp, acc, st));
     } else {
       GM_CHECK_CUDA(launch_k(head_y_fwd_kernel<A>, dim3((B + 7) / 8), dim3(256), 0, st, true, (const float*)logits_y, u, B, K,
                              1.f / c.temperature, inv_bg, y_f32, y_act, Kp, acc));
@@ -1478,6 +1500,9 @@ static int forward_backward_body(gmvae_handle* h, const uint8_t* x_u8, int B, in
       GM_CHECK_CUDA(launch_k(head_y_bwd_row_kernel, dim3(std::max(1, std::min(tc::num_sms(), (B + 127) / 128))), dim3(128), 0, st, true,
                              (const float*)logits_y, (const float*)y_f32, (const float*)dy, B, K, 1.f / c.temperature, inv_bg,
                              reinterpret_cast<bf16*>(dlogits_y), Kp, ey_bias_fused ? h->grads + h->encoder_y.layers[nl - 1].b_off : (float*)nullptr));
+    } else if (K > HEAD_MAXK) {
+      GM_TRY(head_y_wide_bwd<A>(K, logits_y, y_f32, dy, B, 1.f / c.temperature, inv_bg, dlogits_y, Kp,
+                                ey_bias_fused ? h->grads + h->encoder_y.layers[nl - 1].b_off : (float*)nullptr, st));
     } else {
       GM_CHECK_CUDA(launch_k(head_y_bwd_kernel<A>, dim3(std::max(1, std::min(2 * tc::num_sms(), (B + 7) / 8))), dim3(256), 0, st, true,
                              (const float*)logits_y, (const float*)y_f32, (const float*)dy, B, K, 1.f / c.temperature, inv_bg, dlogits_y, Kp,
@@ -1705,8 +1730,12 @@ int gmvae_create(const gmvae_config* cfg, gmvae_handle** out) {
   GM_REQUIRE(cfg->num_hidden >= 0 && cfg->num_hidden <= GMVAE_MAX_HIDDEN_LAYERS, "num_hidden out of range");
   GM_REQUIRE(cfg->data_size > 0 && cfg->latent_size > 0 && cfg->max_batch > 0, "sizes must be positive");
   for (int i = 0; i < cfg->num_hidden; ++i) GM_REQUIRE(cfg->hidden_sizes[i] > 0, "hidden sizes must be positive");
-  if (cfg->model != GMVAE_MODEL_VAE)
-    GM_REQUIRE(cfg->mixture_components >= 1 && cfg->mixture_components <= HEAD_MAXK, "mixture_components must be in [1,128]");
+  if (cfg->model != GMVAE_MODEL_VAE) {
+    // the wide q(y|x) heads serve the GMVAE's objective R; VAE_GMP's prior and objective M's per-component kernels stop at HEAD_MAXK
+    const int kmax = cfg->model == GMVAE_MODEL_GMVAE && cfg->objective == GMVAE_OBJECTIVE_REFERENCE ? HEAD_WIDE_MAXK : HEAD_MAXK;
+    GM_REQUIRE(cfg->mixture_components >= 1 && cfg->mixture_components <= kmax,
+               "mixture_components must be in [1," + std::to_string(kmax) + "]");
+  }
   GM_REQUIRE(cfg->objective == GMVAE_OBJECTIVE_REFERENCE || cfg->model == GMVAE_MODEL_GMVAE, "objective applies to GMVAE only");
   if (cfg->objective == GMVAE_OBJECTIVE_MARGINAL) {
     GM_REQUIRE(cfg->num_hidden >= 1 && cfg->latent_size <= 256, "objective=marginal needs at least one hidden layer and latent_size <= 256");

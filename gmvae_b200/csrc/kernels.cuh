@@ -234,6 +234,124 @@ __global__ void head_y_bwd_kernel(const float* __restrict__ logits, const float*
   }
 }
 
+// ---- q(y|x) head for HEAD_MAXK < K <= HEAD_WIDE_MAXK (GMVAE, objective R) --------------------------
+// The math of head_y_fwd_kernel / head_y_bwd_kernel, one warp per row with MAXK / 32 values per lane.  MAXK (256, 512 or
+// 1024) is the smallest that holds K (engine.cu head_y_wide_fwd / _bwd), so a 129-wide head does not pay for 1024 registers'
+// worth of row.  Objective R only: the Gumbel noise and dy are always present.  Blocks of HEAD_WIDE_THREADS threads.
+constexpr int HEAD_WIDE_MAXK = 1024, HEAD_WIDE_THREADS = 256;
+template <typename ActT, int MAXK>
+__global__ void __launch_bounds__(HEAD_WIDE_THREADS) head_y_wide_fwd_kernel(const float* __restrict__ logits, const float* __restrict__ gum,
+                                                                            int B, int K, float inv_T, float inv_bg, float* __restrict__ y_f32,
+                                                                            ActT* __restrict__ y_act, int ld_yact, float* __restrict__ acc) {
+  constexpr int NI = MAXK / 32;
+  griddep_wait();
+  griddep_launch();
+  __shared__ float scratch[32];
+  const int lane = threadIdx.x & 31;
+  const int row = blockIdx.x * (HEAD_WIDE_THREADS / 32) + (threadIdx.x >> 5);
+  float ent = 0.f;
+  if (row < B) {
+    const float* lr = logits + (int64_t)row * K; const float* gr = gum + (int64_t)row * K;
+    float l[NI], a[NI];
+    float ml = -INFINITY, ma = -INFINITY;
+#pragma unroll
+    for (int i = 0; i < NI; ++i) {
+      const int k = lane + 32 * i;
+      l[i] = -INFINITY; a[i] = -INFINITY;
+      if (k < K) { l[i] = lr[k]; a[i] = (l[i] + gr[k]) * inv_T; }
+      ml = fmaxf(ml, l[i]); ma = fmaxf(ma, a[i]);
+    }
+    ml = warp_max(ml); ma = warp_max(ma);
+    float sl = 0.f, nm = 0.f, sa = 0.f;
+#pragma unroll
+    for (int i = 0; i < NI; ++i)
+      if (lane + 32 * i < K) { if (l[i] == ml) nm += 1.f; else sl += expf(l[i] - ml); sa += expf(a[i] - ma); }
+    sl = warp_sum(sl); nm = warp_sum(nm); sa = warp_sum(sa);
+    const float lo = lse_above_max(sl, nm), inv_sa = 1.f / sa;
+    float* yr = y_f32 + (int64_t)row * K; ActT* ar = y_act + (int64_t)row * ld_yact;
+#pragma unroll
+    for (int i = 0; i < NI; ++i) {
+      const int k = lane + 32 * i;
+      if (k < K) {
+        const float logp = (l[i] - ml) - lo;
+        ent += expf(logp) * logp;
+        const float y = expf(a[i] - ma) * inv_sa;
+        yr[k] = y;
+        ar[k] = from_f32<ActT>(y);
+      } else if (k < ld_yact) {
+        ar[k] = from_f32<ActT>(0.f);
+      }
+    }
+  }
+  const float s = block_sum(ent, scratch);
+  if (threadIdx.x == 0 && s != 0.f) acc_add(acc, ACC_NENT, s * inv_bg);
+}
+
+// Rows are strided over the grid.  With `db` (default mode) each warp sums its rows' stored dl per column in its own slice of
+// shared memory, and the block adds the slices with one global atomic per column; deterministic mode passes null and takes the
+// bias gradient from its fixed-order column sum (engine.cu bias_grad).
+template <typename ActT, int MAXK>
+__global__ void __launch_bounds__(HEAD_WIDE_THREADS) head_y_wide_bwd_kernel(const float* __restrict__ logits, const float* __restrict__ y_f32,
+                                                                            const float* __restrict__ dy, int B, int K, float inv_T, float inv_bg,
+                                                                            ActT* __restrict__ dlogits, int ld_out, float* __restrict__ db) {
+  constexpr int NI = MAXK / 32, WARPS = HEAD_WIDE_THREADS / 32;
+  griddep_wait();
+  griddep_launch();
+  __shared__ float cs[WARPS][MAXK];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  if (db) {
+#pragma unroll
+    for (int i = 0; i < NI; ++i) cs[w][lane + 32 * i] = 0.f;
+  }
+  for (int row = blockIdx.x * WARPS + w; row < B; row += gridDim.x * WARPS) {
+    const float* lr = logits + (int64_t)row * K; const float* yr = y_f32 + (int64_t)row * K; const float* gr = dy + (int64_t)row * K;
+    float l[NI], y[NI], g[NI];
+    float ml = -INFINITY, ydy = 0.f;
+#pragma unroll
+    for (int i = 0; i < NI; ++i) {
+      const int k = lane + 32 * i;
+      l[i] = -INFINITY; y[i] = 0.f; g[i] = 0.f;
+      if (k < K) { l[i] = lr[k]; y[i] = yr[k]; g[i] = gr[k]; }
+      ml = fmaxf(ml, l[i]);
+      ydy += y[i] * g[i];
+    }
+    ml = warp_max(ml); ydy = warp_sum(ydy);
+    float sl = 0.f, nm = 0.f;
+#pragma unroll
+    for (int i = 0; i < NI; ++i)
+      if (lane + 32 * i < K) { if (l[i] == ml) nm += 1.f; else sl += expf(l[i] - ml); }
+    sl = warp_sum(sl); nm = warp_sum(nm);
+    const float lo = lse_above_max(sl, nm);
+    float plogp = 0.f;
+#pragma unroll
+    for (int i = 0; i < NI; ++i)
+      if (lane + 32 * i < K) { const float lp = (l[i] - ml) - lo; plogp += expf(lp) * lp; }
+    plogp = warp_sum(plogp);
+    ActT* orow = dlogits + (int64_t)row * ld_out;
+#pragma unroll
+    for (int i = 0; i < NI; ++i) {
+      const int k = lane + 32 * i;
+      if (k < K) {
+        const float lp = (l[i] - ml) - lo;
+        const ActT o = from_f32<ActT>(y[i] * (g[i] - ydy) * inv_T + expf(lp) * (lp - plogp) * inv_bg);
+        orow[k] = o;
+        if (db) cs[w][k] += to_f32<ActT>(o);
+      } else if (k < ld_out) {
+        orow[k] = from_f32<ActT>(0.f);
+      }
+    }
+  }
+  if (db) {
+    __syncthreads();
+    for (int k = threadIdx.x; k < K; k += HEAD_WIDE_THREADS) {
+      float t = 0.f;
+#pragma unroll
+      for (int j = 0; j < WARPS; ++j) t += cs[j][k];
+      if (t != 0.f) atomicAdd(db + k, t);
+    }
+  }
+}
+
 // ---- q(z|.) head, forward (base.py:69-70; gmvae.py:248,258; vae.py:171,181) ---------------------
 // enc_out = [mu | raw] (B x 2Z).  sigma = max(softplus(raw + c), sigma_min); z = mu + sigma eps.
 // KL accumulator gets log q(z) - log p(z) summed over the batch, divided by the global batch:

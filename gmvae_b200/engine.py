@@ -27,7 +27,8 @@ class Engine:
                  temperature: float = 1.0, learning_rate: float = 1e-3, beta1: float = 0.9,
                  beta2: float = 0.999, epsilon: float = 1e-8, device: Optional[int] = None,
                  seed: Optional[int] = None, init: bool = True, deterministic: bool = False):
-        """deterministic=True: bitwise-reproducible training steps (gmvae_config::deterministic, DESIGN.md section 9)."""
+        """deterministic=True: bitwise-reproducible training steps (gmvae_config::deterministic, DESIGN.md section 9).
+        mixture_components: up to 1024 for the GMVAE under objective "reference", up to 128 for VAE_GMP and "marginal"."""
         if not torch.cuda.is_available():
             raise RuntimeError("gmvae_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = _lib.load()

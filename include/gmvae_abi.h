@@ -58,7 +58,7 @@ typedef struct gmvae_config {
   int32_t precision;          /* GMVAE_PRECISION_* */
   int32_t data_size;          /* 784 */
   int32_t latent_size;        /* --latent_size */
-  int32_t mixture_components; /* --mixture_components */
+  int32_t mixture_components; /* --mixture_components: [1,1024] for the GMVAE under objective R, [1,128] for VAE_GMP and objective M */
   int32_t num_hidden;         /* len(fcnet_hidden_sizes) */
   int32_t hidden_sizes[GMVAE_MAX_HIDDEN_LAYERS];
   int32_t max_batch;          /* largest per-device batch this handle will see */
